@@ -3,7 +3,7 @@
 calibration tokens (configs[1]; YAML = configs/gptq_w_only.yml, the schema of the reference's
 configs/quantization/methods/GPTQ/gptq_w_only.yml).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A STEP = GPTQ calibration of ONE decoder block (7 linears: RTN seed qparams, Hessians over the
 full calibration set, Cholesky, column sweep, fake-quant forward that feeds the next block).
@@ -25,6 +25,10 @@ does it per batch); total work fixed => "scaling": "strong".
 the GPU box) on the host cores: every step is the same workload — one decoder block through the
 reference's schedule at the real shapes — on a bounded sample (see REF_SAMPLE), and the reported
 value is extrapolated to the full calibration set with stated rules.
+
+--dump-outputs DIR: after the timed steps, write what the last device-resident step produced
+(block_outputs) to DIR/<name>.npy, so that two builds can be compared output for output on the
+same seeded inputs.
 """
 import argparse
 import json
@@ -275,6 +279,9 @@ def run_ours(args):
     TIMER.enabled = False
     clocks = sampler.stop()
     loss_probe = algo.layer_loss(f'{W}.self_attn.q_proj') if K > 0 else None
+    dump = None
+    if args.dump_outputs and rank == 0 and K > 0:
+        dump = block_outputs(algo, model, blocks[W + K - 1], W + K - 1)
     del algo, model, blocks
     torch.cuda.empty_cache()
 
@@ -401,7 +408,46 @@ def run_ours(args):
         'cpu_baseline': cpu,
         'check': {'q_proj_loss_first_timed_block': loss_probe, 'dominant_span': dom},
     }
+    if dump is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(args.dump_outputs, f'{name}.npy'), arr)
     emit(line)
+
+
+DUMP_BYTES = 64 << 20            # all arrays of --dump-outputs together
+DUMP_MAX_ELEMS = 1 << 19         # per array; larger arrays are reduced to a seeded sample
+
+
+def block_outputs(algo, model, block, idx):
+    """What block_opt hands its caller for block `idx`, as host float arrays: per linear the
+    GPTQ-compensated fp32 weight, the fake-quant weight the next forward uses, the group scales /
+    zeros, the act-order permutation and the per-row losses; and the block's output, which is the
+    next block's calibration input.  An array above the per-array share of DUMP_BYTES is reduced
+    to the same seeded choice of elements in every run (integers go to float64, exact; the rest to
+    float32)."""
+    arrays = {}
+    for name, m in model.get_block_linears(block).items():
+        for buf in ('weight', 'tmp_weight', 'buf_scales', 'buf_zeros', 'buf_perm'):
+            t = getattr(m, buf, None)
+            if torch.is_tensor(t):
+                arrays[f'{name}.{buf}'] = t
+        arrays[f'{name}.losses'] = algo.losses[f'{idx}.{name}']
+    x = algo.input.get('stacked')
+    arrays['block_output'] = x if x is not None else torch.cat(algo.input['data'])
+    share = DUMP_BYTES // len(arrays)
+    out = {}
+    for name, t in arrays.items():
+        flat = t.detach().reshape(-1)
+        dt = torch.float32 if t.is_floating_point() else torch.float64
+        n = min(DUMP_MAX_ELEMS, share // dt.itemsize)
+        if flat.numel() > n:
+            g = torch.Generator().manual_seed(flat.numel())
+            idx_s = torch.randint(flat.numel(), (n,), generator=g).sort().values
+            flat = flat[idx_s.to(flat.device)]
+        out[name] = flat.to(dt).cpu().numpy().reshape(t.shape if flat.numel() == t.numel() else -1)
+    return out
 
 
 # ---------------------------------------------------------------------------------- CPU baseline
@@ -578,7 +624,11 @@ def main():
     ap.add_argument('--model', default=MODEL)
     ap.add_argument('--samples', type=int, default=N_SAMPLES)
     ap.add_argument('--seq-len', dest='seq_len', type=int, default=SEQ_LEN)
+    ap.add_argument('--dump-outputs', dest='dump_outputs', metavar='DIR', default=None,
+                    help='write the last timed step\'s results to DIR/<name>.npy (at most 64 MiB)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs dumps the CUDA path; the reference arm runs a sampled CPU block')
     if args.impl == 'reference':
         return run_reference(args)
     if not torch.cuda.is_available():

@@ -191,8 +191,31 @@ def run_case(name, quant, dtype, n_calib, calib_len, bs, n_eval, eval_len, seed=
           f'size {os.path.getsize(os.path.join(OUT, f"e2e_{name}.pt")) / 1e6:.1f} MB')
 
 
+CPU_THREADS = 8
+
+
+def gptq_cpu_losses():
+    """The reference's per-layer GPTQ Losses.sum() on the e2e_gptq_llama inputs, run on this host's
+    CPU torch build with CPU_THREADS threads -> e2e_gptq_llama_cpu_losses.json, the expected values
+    of tests/test_oracle_golden.py::test_block_oracle_reproduces_reference_pipeline.  bf16 CPU GEMMs
+    round differently between CPU builds and thread counts, and GPTQ carries that from block 0's
+    quantised output into block 1, so the file records the build and thread count it came from."""
+    import json
+    torch.set_num_threads(CPU_THREADS)
+    out = run_case('gptq_llama', GPTQ_QUANT, torch.bfloat16, 16, 128, 1, 8, 128, save=False)
+    stored = torch.load(os.path.join(OUT, 'e2e_gptq_llama.pt'), weights_only=False)
+    assert torch.equal(out['calib_ids'], stored['calib_ids'])
+    doc = dict(what='reference GPTQ run_block_loop on the e2e_gptq_llama inputs, CPU: per-layer Losses.sum()',
+               torch=torch.__version__, cpu_capability=torch.backends.cpu.get_cpu_capability(),
+               threads=CPU_THREADS, losses=out['losses'])
+    path = os.path.join(OUT, 'e2e_gptq_llama_cpu_losses.json')
+    with open(path, 'w') as fh:
+        json.dump(doc, fh, indent=1)
+    print(path, len(out['losses']), 'layers')
+
+
 if __name__ == '__main__':
-    which = sys.argv[1:] or ['gptq', 'awq', 'awq_gqa', 'rtn', 'sq', 'hqq', 'spqr']
+    which = sys.argv[1:] or ['gptq', 'awq', 'awq_gqa', 'rtn', 'sq', 'hqq', 'spqr', 'gptq_cpu']
     if 'hqq' in which:
         run_case('hqq_llama', HQQ_QUANT, torch.bfloat16, 4, 64, 1, 8, 128)
     if 'sq' in which:
@@ -211,3 +234,5 @@ if __name__ == '__main__':
         run_case('spqr_llama', SPQR_QUANT, torch.bfloat16, 16, 128, 1, 8, 128)
     if 'rtn' in which:
         run_case('rtn_llama', RTN_QUANT, torch.bfloat16, 4, 64, 1, 8, 128)
+    if 'gptq_cpu' in which:
+        gptq_cpu_losses()

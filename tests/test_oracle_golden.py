@@ -187,24 +187,37 @@ def test_awq_search_and_clip(golden_dir):
 
 def test_block_oracle_reproduces_reference_pipeline(golden_dir):
     """oracle/block_oracle.py (the five-forward GPTQ schedule of one decoder block, also the CPU
-    arm of bench.py) against the reference's own end-to-end run on the tiny Llama
-    (tests/golden/e2e_gptq_llama.pt): per-layer Losses.sum() of BOTH blocks — block 1 only matches
-    if block 0's quantised output (the quant_out pass) is right."""
+    arm of bench.py) against the reference's own end-to-end run on the tiny Llama (inputs:
+    tests/golden/e2e_gptq_llama.pt): per-layer Losses.sum() of BOTH blocks — block 1 only matches
+    if block 0's quantised output (the quant_out pass) is right.
+
+    bf16 CPU GEMMs round differently between CPU builds and thread counts, and GPTQ carries that
+    from block 0 into block 1 at the 1e-2 level (as far as the reference's sdpa and eager runs
+    differ).  The expected losses (tests/golden/e2e_gptq_llama_cpu_losses.json) therefore come from
+    a CPU run of the reference at a recorded thread count, and the oracle runs at that count."""
+    import json
     from oracle import block_oracle as bo
     d = _load(golden_dir, 'e2e_gptq_llama.pt')
+    with open(os.path.join(golden_dir, 'e2e_gptq_llama_cpu_losses.json')) as fh:
+        ref_run = json.load(fh)
     sd = _load(golden_dir, d['init'])['sd0']
     x = [torch.nn.functional.embedding(d['calib_ids'][i:i + 1], sd['model.embed_tokens.weight'])
          for i in range(d['calib_ids'].shape[0])]
-    for blk in range(2):
-        W = {n: sd[f'model.layers.{blk}.{"self_attn" if "proj" in n and n[0] in "qkvo" else "mlp"}.{n}.weight']
-             for n in bo.LINEARS}
-        W['ln1'] = sd[f'model.layers.{blk}.input_layernorm.weight']
-        W['ln2'] = sd[f'model.layers.{blk}.post_attention_layernorm.weight']
-        x, _, info = bo.gptq_block(W, x, heads=4, kv_heads=2)
-        for n in bo.LINEARS:
-            mod = 'self_attn' if n in ('q_proj', 'k_proj', 'v_proj', 'o_proj') else 'mlp'
-            ref = d['losses'][f'{blk}.{mod}.{n}']
-            assert info[n]['loss'] == pytest.approx(ref, rel=2e-3), (blk, n, info[n]['loss'], ref)
+    threads = torch.get_num_threads()
+    torch.set_num_threads(ref_run['threads'])
+    try:
+        for blk in range(2):
+            W = {n: sd[f'model.layers.{blk}.{"self_attn" if "proj" in n and n[0] in "qkvo" else "mlp"}.{n}.weight']
+                 for n in bo.LINEARS}
+            W['ln1'] = sd[f'model.layers.{blk}.input_layernorm.weight']
+            W['ln2'] = sd[f'model.layers.{blk}.post_attention_layernorm.weight']
+            x, _, info = bo.gptq_block(W, x, heads=4, kv_heads=2)
+            for n in bo.LINEARS:
+                mod = 'self_attn' if n in ('q_proj', 'k_proj', 'v_proj', 'o_proj') else 'mlp'
+                ref = ref_run['losses'][f'{blk}.{mod}.{n}']
+                assert info[n]['loss'] == pytest.approx(ref, rel=2e-3), (blk, n, info[n]['loss'], ref)
+    finally:
+        torch.set_num_threads(threads)
 
 
 def test_range_oracle_matches_reference(golden_dir):
