@@ -356,14 +356,33 @@ int llmc_fp8_quant(const void* w, int64_t rows, int64_t cols, int dtype, int64_t
  *       (fp32, written to scales [ceil(M/block), ceil(N/block)]), q = fp8(x.float() / scale);
  *       out_mode 0 scales only | 1 QDQ (`dtype`) | 2 fp8 bytes.
  *   llmc_fp8_block_dequant  weight_cast_to_bf16 (quant.py:18-29): bf16(fp8.float() * scale_inv).
- *   (The reference's Triton act_quant / fp8_gemm pair, kernel.py:31-53, 141-242, is not built: the
- *   forward of LlmcFp8Linear dequantises once and runs the bf16 tcgen05 GEMM, the reference's own
- *   non-Triton branch, module_utils.py:171-178.)
+ *   The forward on these checkpoints is the block-scaled pair below (llmc_fp8_act_quant +
+ *   llmc_fp8_gemm); LlmcFp8Linear keeps the dequantise-once branch as its default.
  * ------------------------------------------------------------------------------------ */
 int llmc_fp8_block_quant(const void* w, int64_t M, int64_t N, int dtype, int block, int e5m2,
                          float* scales, int out_mode, void* out, void* stream);
 int llmc_fp8_block_dequant(const void* w_fp8, int64_t M, int64_t N, int block, int e5m2,
                            const float* scale_inv, void* out_bf16, void* stream);
+
+/* ------------------------------------------------------------------------------------
+ * K7-fp8  block-scaled FP8 forward (csrc/gemm_fp8.cu) — the reference's Triton pair
+ *   act_quant / fp8_gemm (kernel.py:31-53, 141-242) behind block_wise_fp8_forward_func.
+ *   llmc_fp8_act_quant  x [M, K] (dtype fp32 / fp16 / bf16, contiguous), K % 128 == 0:
+ *       per 1 x 128 block s = absmax / 448, y = e4m3(x / s), both divisions `div.full.f32` and
+ *       the conversion `cvt.rn.satfinite.e4m3x2.f32` as in the reference's compiled kernel.
+ *       y [M, K] e4m3 bytes, s [M, K/128] fp32.  An all-zero block gives s = 0 and NaN codes.
+ *   llmc_fp8_gemm  C[M, N] = sum_kb (A_kb . B_kb^T) * a_s[m, kb] * b_s[n / 128, kb]
+ *       A [M, K] and B [N, K] e4m3 (K-major), a_s [M, K/128], b_s [ceil(N/128), K/128] fp32,
+ *       K % 128 == 0 (weight blocks are 128 wide whatever block size the activations used).
+ *       fp32 accumulation, per K-block promotion acc = fma(dot * a_s, b_s, acc), one rounding to
+ *       out_dtype (fp32 / fp16 / bf16).  bias (fp32 or bf16, may be NULL) requires a bf16
+ *       output and is added as `y += bias` after that rounding: bf16(float(y) + float(bias)).
+ * ------------------------------------------------------------------------------------ */
+int llmc_fp8_act_quant(const void* x, int64_t M, int64_t K, int dtype, void* y, float* s,
+                       void* stream);
+int llmc_fp8_gemm(const void* a, const float* a_s, const void* b, const float* b_s,
+                  const void* bias, int bias_dtype, void* c, int out_dtype, int64_t M, int64_t N,
+                  int64_t K, void* stream);
 
 /* ------------------------------------------------------------------------------------
  * Block-forward glue (csrc/block_ops.cu) for F2 block_forward

@@ -72,6 +72,9 @@ SIGNATURES = {
                                c_vp, c_vp]),
     'llmc_fp8_block_quant': (c_int, [c_vp, c_i64, c_i64, c_int, c_int, c_int, c_vp, c_int, c_vp, c_vp]),
     'llmc_fp8_block_dequant': (c_int, [c_vp, c_i64, c_i64, c_int, c_int, c_vp, c_vp, c_vp]),
+    'llmc_fp8_act_quant': (c_int, [c_vp, c_i64, c_i64, c_int, c_vp, c_vp, c_vp]),
+    'llmc_fp8_gemm': (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_i64, c_i64, c_i64,
+                              c_vp]),
     'llmc_gemm_w4a16': (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64,
                                 c_int, c_vp]),
     'llmc_gemm_w8a16': (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64,

@@ -357,6 +357,26 @@ int encode_tmap_2d_b16(CUtensorMap* out, const void* base, uint64_t rows, uint64
   return LLMC_OK;
 }
 
+int encode_tmap_2d_u8(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
+                      uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols) {
+  PFN_tmapEncodeTiled fn = get_encode_fn();
+  if (!fn) return LLMC_ECUDA;
+  cuuint64_t dims[2] = {cols, rows};
+  cuuint64_t strides[1] = {ld_elems};
+  cuuint32_t box[2] = {box_cols, box_rows};
+  cuuint32_t estr[2] = {1, 1};
+  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base), dims, strides,
+                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    set_last_error("cuTensorMapEncodeTiled(u8) failed with CUresult %d (rows %llu cols %llu ld %llu)",
+                   (int)r, (unsigned long long)rows, (unsigned long long)cols,
+                   (unsigned long long)ld_elems);
+    return LLMC_ECUDA;
+  }
+  return LLMC_OK;
+}
+
 int encode_tmap_2d_f32(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
                        uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols, int atom32b) {
   PFN_tmapEncodeTiled fn = get_encode_fn();

@@ -182,6 +182,43 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64
       : "memory");
 }
 
+// Instruction descriptor for kind::f8f6f4 with E4M3 x E4M3 -> F32, both operands K-major.
+// Same field layout as kind::f16; the A/B format code 0 means E4M3 under this kind.
+__host__ __device__ constexpr uint32_t make_idesc_e4m3(int M, int N) {
+  return (1u << 4) | (static_cast<uint32_t>(N >> 3) << 17) | (static_cast<uint32_t>(M >> 4) << 24);
+}
+
+// D[tmem] (+)= A[smem] * B[smem] for 8-bit operands (K = 32 per instruction), ONE thread.
+__device__ __forceinline__ void umma_f8f6f4(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc,
+                                            uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+
+// Packed fp32 pair arithmetic (sm_100): (c0, c1) = fma((d0, d1) * sa, sb, (c0, c1)), with the
+// product d * sa rounded on its own (mul.rn then fma.rn, never contracted into one fma).
+__device__ __forceinline__ void promote2(float& c0, float& c1, float d0, float d1, float sa,
+                                         float sb) {
+  asm("{\n"
+      ".reg .b64 d, a, b, c;\n"
+      "mov.b64 d, {%2, %3};\n"
+      "mov.b64 a, {%4, %4};\n"
+      "mov.b64 b, {%5, %5};\n"
+      "mov.b64 c, {%0, %1};\n"
+      "mul.rn.f32x2 d, a, d;\n"
+      "fma.rn.f32x2 c, d, b, c;\n"
+      "mov.b64 {%0, %1}, c;\n"
+      "}\n"
+      : "+f"(c0), "+f"(c1)
+      : "f"(d0), "f"(d1), "f"(sa), "f"(sb));
+}
+
 }  // namespace tc
 
 // ---- host: tensor-map encoding through the driver entry point ---------------------------------
@@ -189,5 +226,8 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64
 // 128-byte swizzle (box_cols * 2 must be 128).
 int encode_tmap_2d_b16(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
                        uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols);
+// The same for 1-byte elements (fp8): box_cols must be 128.
+int encode_tmap_2d_u8(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
+                      uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols);
 
 }  // namespace llmc

@@ -5,14 +5,53 @@ VllmRealQuantLinear (:762-876) + aliases (:879-933), AutoawqRealQuantLinear (:93
 MlcllmRealQuantLinear (:1068-1084), and the type maps (:1087-1138).  Same `.new(...)`
 factories, buffer names and `buf_*` hand-off; the forward GEMM and the packers run in
 libllmc_b200.so.
+
+128 x 128 block-FP8 weights (DeepSeek-V3 / R1 checkpoints) have two forwards, which are two of
+the reference's semantics rather than two implementations of one result:
+  * dequantise-once (the reference on pre-Hopper GPUs, module_utils.py:163-167): the weight is
+    cast to bf16 once and every later forward is a bf16 GEMM on it;
+  * block-scaled (the reference on Hopper and newer, :40-45, 151-161): block_wise_fp8_forward_func
+    quantises the activations per 1 x 128 block and runs the FP8 GEMM with per-block scale
+    promotion (csrc/gemm_fp8.cu), keeping the weight in fp8.
+OriginFloatLinear, FakeQuantLinear and EffcientFakeQuantLinear built from an fp8 module always take
+the block-scaled forward, as the reference does.  LlmcFp8Linear takes it when
+USE_FP8GEMM_TRITON_KERNEL is true (the reference's switch, named after its Triton kernels; here it
+selects the CUDA pair), initialised from the environment variable LLMC_B200_FP8_GEMM ('1' = on)
+and off by default, so LlmcFp8Linear keeps dequantising once unless asked.
 """
+import os
 from functools import partial
 
 import torch
 import torch.nn as nn
 
 from ._lib import call, dtype_enum, ptr, require_cuda, stream_ptr
+from .kernel import act_quant, fp8_gemm, fp8_gemm_out
 from .prof import TIMER
+
+USE_FP8GEMM_TRITON_KERNEL = os.environ.get('LLMC_B200_FP8_GEMM', '0') == '1'
+
+
+def block_wise_fp8_forward_func(x, w, w_scale, block_size, bias):
+    """module_utils.py:40-45: act_quant -> fp8_gemm -> .to(bf16) -> `y += bias`.  When
+    fp8_gemm's default-dtype result reaches bf16 in one rounding (default dtype fp32 or bf16), the
+    bf16 cast and the bias add run in the GEMM's epilogue, with the same two roundings."""
+    x, scale = act_quant(x, block_size)
+    if torch.get_default_dtype() in (torch.float32, torch.bfloat16) and (
+            bias is None or bias.dtype in (torch.float32, torch.bfloat16)):
+        return fp8_gemm_out(x, scale, w, w_scale, torch.bfloat16, bias)
+    y = fp8_gemm(x, scale, w, w_scale).to(torch.bfloat16)
+    if bias is not None:
+        y += bias
+    return y
+
+
+def _fp8_source(dst, ori_module):
+    """The reference's fp8 branch of the wrappers' __init__ (e.g. module_utils.py:413-418)."""
+    dst.fp8_forward = dst.weight.dtype == torch.float8_e4m3fn
+    if dst.fp8_forward:
+        dst.weight_scale_inv = ori_module.weight_scale_inv
+        dst.block_size = ori_module.block_size
 
 
 def linear_forward(x, weight, bias=None):
@@ -98,9 +137,13 @@ class OriginFloatLinear(nn.Module):
         if getattr(self, 'buf_rotate', False):
             raise NotImplementedError('online rotation (QuaRot) is out of scope (SURVEY §2 #12)')
         self.buf_rotate = False
+        _fp8_source(self, ori_module)
 
     @torch.no_grad()
     def forward(self, x):
+        if self.fp8_forward:
+            return block_wise_fp8_forward_func(x, self.weight, self.weight_scale_inv, self.block_size,
+                                               self.bias)
         return linear_forward(x, self.weight, self.bias)
 
     @classmethod
@@ -115,13 +158,15 @@ class OriginFloatLinear(nn.Module):
     def __repr__(self):
         return (f'OriginFloatLinear(in_features={self.in_features},'
                 f'out_features={self.out_features}, bias={self.bias is not None},'
-                f'online_rotate={self.buf_rotate})')
+                f'online_rotate={self.buf_rotate},'
+                f'fp8_forward={self.fp8_forward})')
 
 
 class LlmcFp8Linear(nn.Module):
     """module_utils.py:130-191 — holder of a 128x128 block-FP8 checkpoint weight (`weight` fp8 +
-    `weight_scale_inv` fp32 [ceil(out/bs), ceil(in/bs)]).  Forward = the reference's non-Triton branch
-    (:171-178): dequantise ONCE to bf16 (llmc_fp8_block_dequant) and run the tcgen05 GEMM."""
+    `weight_scale_inv` fp32 [ceil(out/bs), ceil(in/bs)]).  Forward: with USE_FP8GEMM_TRITON_KERNEL
+    the block-scaled FP8 GEMM on the fp8 weight (:153-161); otherwise the reference's other branch
+    (:162-167), dequantise ONCE to bf16 (llmc_fp8_block_dequant) and run the tcgen05 GEMM."""
 
     def __init__(self, in_features, out_features, bias, block_size):
         super().__init__()
@@ -138,6 +183,9 @@ class LlmcFp8Linear(nn.Module):
     @torch.no_grad()
     def forward(self, x):
         if self.weight.data.dtype == torch.float8_e4m3fn:
+            if USE_FP8GEMM_TRITON_KERNEL:
+                return block_wise_fp8_forward_func(x, self.weight, self.weight_scale_inv,
+                                                   self.block_size, self.bias)
             from .quant_float import weight_cast_to_bf16
             self.weight.data = weight_cast_to_bf16(self.weight.data, self.weight_scale_inv.data,
                                                    self.block_size)
@@ -152,7 +200,7 @@ class LlmcFp8Linear(nn.Module):
         return (f'LlmcFp8Linear(in_features={self.in_features}, out_features={self.out_features}, '
                 f'bias={self.bias is not None}, weight_shape={self.weight.shape}, '
                 f'weight_dtype={self.weight.dtype}, block_size={self.block_size}, '
-                'use_fp8gemm_triton_kernel=False)')
+                f'use_fp8gemm_triton_kernel={USE_FP8GEMM_TRITON_KERNEL})')
 
 
 class FakeQuantLinear(nn.Module):
@@ -172,9 +220,7 @@ class FakeQuantLinear(nn.Module):
         if getattr(self, 'buf_rotate', False):
             raise NotImplementedError('online rotation (QuaRot) is out of scope (SURVEY §2 #12)')
         self.buf_rotate = False
-        if self.weight.data.dtype == torch.float8_e4m3fn:
-            raise NotImplementedError('fp8 checkpoints (LlmcFp8Linear) are a SURVEY §8(f) row')
-        self.fp8_forward = False
+        _fp8_source(self, ori_module)
         self.dynamic_quant_weight = False
         self.dynamic_quant_tmp_weight = False
 
@@ -189,6 +235,10 @@ class FakeQuantLinear(nn.Module):
             self.tmp_bias = self.bias
         elif self.dynamic_quant_tmp_weight:
             self.tmp_weight = self.w_qdq(self)
+        if self.fp8_forward:
+            # the reference evaluates (and caches) w_qdq above, then runs on the fp8 weight (:638-641)
+            return block_wise_fp8_forward_func(x, self.weight, self.weight_scale_inv, self.block_size,
+                                               self.bias)
         return linear_forward(x, self.tmp_weight, self.tmp_bias)
 
     @classmethod
@@ -262,6 +312,10 @@ class EffcientFakeQuantLinear(nn.Module):
         if getattr(self, 'buf_rotate', False):
             raise NotImplementedError('online rotation (QuaRot) is out of scope (SURVEY §2 #12)')
         self.buf_rotate = False
+        if packed is None:
+            _fp8_source(self, ori_module)
+        else:
+            self.fp8_forward = False
 
     def __getattr__(self, name):
         if name == 'weight' and self.__dict__.get('packed', False):
@@ -285,6 +339,9 @@ class EffcientFakeQuantLinear(nn.Module):
     def forward(self, x):
         if self.a_qdq is not None:
             x = self.a_qdq(x, self)
+        if self.fp8_forward:
+            return block_wise_fp8_forward_func(x, self.weight, self.weight_scale_inv, self.block_size,
+                                               self.bias)
         if self.packed:
             return linear_forward_w4(x, self.qweight, self.qscales_t, self.qzeros_t, self.q_group, self.bias,
                                      bits=self.q_bits, qparams_t=True)
@@ -293,10 +350,10 @@ class EffcientFakeQuantLinear(nn.Module):
     @classmethod
     @torch.no_grad()
     def new(cls, module, w_qdq, a_qdq, debug_print={}):
-        import os
         packer = getattr(w_qdq, 'packed', None)
         packed = None
-        if packer is not None and os.environ.get('LLMC_B200_FUSED_DEQUANT', '1') != '0':
+        fp8 = module.weight.dtype == torch.float8_e4m3fn     # fp8 checkpoints: never packed
+        if packer is not None and not fp8 and os.environ.get('LLMC_B200_FUSED_DEQUANT', '1') != '0':
             packed = packer(module)
         weight = w_qdq(module) if packed is None else None
         bias = module.bias.data if getattr(module, 'bias', None) is not None else None
@@ -313,7 +370,8 @@ class EffcientFakeQuantLinear(nn.Module):
                 f'out_features={self.out_features}, bias={self.bias is not None},'
                 f'weight_quant={self.w_qdq_name},'
                 f'act_quant={self.a_qdq_name},'
-                f'online_rotate={self.buf_rotate})')
+                f'online_rotate={self.buf_rotate},'
+                f'fp8_forward={self.fp8_forward})')
 
 
 def _cfg_get(cfg, key, default=None):
