@@ -17,7 +17,7 @@ LIB_PATH = os.path.join(HERE, LIB_NAME)
 
 NVCC_FLAGS = [
     '-gencode', 'arch=compute_100a,code=sm_100a',
-    '-O3', '-std=c++17', '-lineinfo',
+    '-O3', '-std=c++20', '-lineinfo',
     '-Xcompiler', '-fPIC',
     '--expt-relaxed-constexpr',
     '-cudart', 'static',

@@ -11,26 +11,9 @@
 #include <vector>
 
 #include "tc.cuh"
+#include "tf32.cuh"
 
 namespace llmc {
-
-int tf32x3_update(const float* Ahi, const float* Alo, int a_mn, int64_t lda, const float* Bhi,
-                  const float* Blo, int b_mn, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                  int64_t N, int K, int mode, int tri, int64_t row_off, int64_t col_off,
-                  float* Chi, float* Clo, cudaStream_t st);
-int tf32x3_update_ex(const float* Ahi, const float* Alo, int a_mn, int64_t lda, const float* Bhi,
-                     const float* Blo, int b_mn, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                     int64_t N, int K, int mode, int tri, int64_t row_off, int64_t col_off,
-                     float* Chi, float* Clo, int64_t split_rows, int64_t split_cols,
-                     cudaStream_t st);
-int tf32x3_update_grid(const float* Ahi, const float* Alo, int a_mn, int64_t lda, const float* Bhi,
-                       const float* Blo, int b_mn, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                       int64_t N, int K, int mode, int tri, int64_t row_off, int64_t col_off,
-                       float* Chi, float* Clo, int64_t split_rows, int64_t split_cols,
-                       int one_tile_per_cta, cudaStream_t st);
-int split_tf32(const float* x, int64_t rows, int64_t cols, int64_t ld, float* hi, float* lo,
-               int64_t ld_out, cudaStream_t st);
-
 namespace ch {
 
 constexpr int NB = 128;
@@ -529,10 +512,12 @@ extern "C" int llmc_chol_inv_upper(float* A, int64_t C, void* workspace, int64_t
         if (sidx > 0 && k0 == sp0 + NB)      // columns sp0+128.. of this super-panel come from A' of the previous one
           LLMC_CHECK_CUDA(cudaStreamWaitEvent(hi, evA[sidx - 1], 0));
         // G[k0:, k0:k0+nb] -= L[k0:, sp0:k0] L[k0:k0+nb, sp0:k0]^T ; emits the split of the block
-        if (int rc = tf32x3_update_ex(Lhi + k0 * n + sp0, Llo + k0 * n + sp0, 0, n, Lhi + k0 * n + sp0,
-                                      Llo + k0 * n + sp0, 0, n, G + k0 * n + k0, n, n - k0, nb,
-                                      static_cast<int>(k0 - sp0), 0, 0, 0, 0, Lhi + k0 * n + k0,
-                                      Llo + k0 * n + k0, INT64_MAX, INT64_MAX, hi))
+        if (int rc = tf32x3_update({.Ahi = Lhi + k0 * n + sp0, .Alo = Llo + k0 * n + sp0, .lda = n,
+                                    .Bhi = Lhi + k0 * n + sp0, .Blo = Llo + k0 * n + sp0, .ldb = n,
+                                    .C = G + k0 * n + k0, .ldc = n, .M = n - k0, .N = nb,
+                                    .K = static_cast<int>(k0 - sp0), .mode = 0,
+                                    .Chi = Lhi + k0 * n + k0, .Clo = Llo + k0 * n + k0},
+                                   hi))
           return rc;
       }
       diag_kernel_v2<<<1, 256, diag_smem, hi>>>(G, n, k0, nb, Y, Yhi, Ylo, info);
@@ -545,7 +530,10 @@ extern "C" int llmc_chol_inv_upper(float* A, int64_t C, void* workspace, int64_t
       if (m > 0) {
         if (kb == 0)
           if (int rc = split_tf32(P, m, nb, n, Ph, Pl, n, hi)) return rc;
-        if (int rc = tf32x3_update(Ph, Pl, 0, n, Xh, Xl, 0, n, P, n, m, nb, nb, 1, 0, 0, 0, Ph, Pl, hi))
+        if (int rc = tf32x3_update({.Ahi = Ph, .Alo = Pl, .lda = n, .Bhi = Xh, .Blo = Xl, .ldb = n,
+                                    .C = P, .ldc = n, .M = m, .N = nb, .K = nb, .mode = 1,
+                                    .Chi = Ph, .Clo = Pl},
+                                   hi))
           return rc;
       }
       LLMC_CHECK_CUDA(cudaEventRecord(ev[kb], hi));        // L panel kb, Y_kk final
@@ -557,25 +545,33 @@ extern "C" int llmc_chol_inv_upper(float* A, int64_t C, void* workspace, int64_t
         const int64_t w1 = (n - sp1) < NB ? (n - sp1) : NB;
         // chain: the next column block (also waits for what earlier bulk pieces wrote there)
         if (sidx > 0) LLMC_CHECK_CUDA(cudaStreamWaitEvent(hi, evA[sidx - 1], 0));
-        if (int rc = tf32x3_update_ex(Ah, Al, 0, n, Ah, Al, 0, n, G + sp1 * n + sp1, n, n - sp1, w1, kk, 0,
-                                      0, 0, 0, Lhi + sp1 * n + sp1, Llo + sp1 * n + sp1, INT64_MAX,
-                                      INT64_MAX, hi))
+        if (int rc = tf32x3_update({.Ahi = Ah, .Alo = Al, .lda = n, .Bhi = Ah, .Blo = Al, .ldb = n,
+                                    .C = G + sp1 * n + sp1, .ldc = n, .M = n - sp1, .N = w1,
+                                    .K = kk, .mode = 0,
+                                    .Chi = Lhi + sp1 * n + sp1, .Clo = Llo + sp1 * n + sp1},
+                                   hi))
           return rc;
         // bulk: A' = columns [sp1+128, sp1+128+spw), then B = the rest; lower tiles only
         LLMC_CHECK_CUDA(cudaStreamWaitEvent(bulk, ev[kb], 0));
         const int64_t ca = sp1 + NB;
         const int64_t cb = (ca + spw < n) ? ca + spw : n;
         if (ca < n) {
-          if (int rc = tf32x3_update_grid(Ah, Al, 0, n, Lhi + ca * n + sp0, Llo + ca * n + sp0, 0, n,
-                                          G + sp1 * n + ca, n, n - sp1, cb - ca, kk, 0, 1, sp1, ca,
-                                          nullptr, nullptr, 0, 0, 1, bulk))
+          if (int rc = tf32x3_update({.Ahi = Ah, .Alo = Al, .lda = n,
+                                      .Bhi = Lhi + ca * n + sp0, .Blo = Llo + ca * n + sp0, .ldb = n,
+                                      .C = G + sp1 * n + ca, .ldc = n, .M = n - sp1, .N = cb - ca,
+                                      .K = kk, .mode = 0, .tri = 1, .row_off = sp1, .col_off = ca,
+                                      .one_tile_per_cta = 1},
+                                     bulk))
             return rc;
         }
         LLMC_CHECK_CUDA(cudaEventRecord(evA[sidx], bulk));
         if (cb < n) {
-          if (int rc = tf32x3_update_grid(Ah, Al, 0, n, Lhi + cb * n + sp0, Llo + cb * n + sp0, 0, n,
-                                          G + sp1 * n + cb, n, n - sp1, n - cb, kk, 0, 1, sp1, cb,
-                                          nullptr, nullptr, 0, 0, 1, bulk))
+          if (int rc = tf32x3_update({.Ahi = Ah, .Alo = Al, .lda = n,
+                                      .Bhi = Lhi + cb * n + sp0, .Blo = Llo + cb * n + sp0, .ldb = n,
+                                      .C = G + sp1 * n + cb, .ldc = n, .M = n - sp1, .N = n - cb,
+                                      .K = kk, .mode = 0, .tri = 1, .row_off = sp1, .col_off = cb,
+                                      .one_tile_per_cta = 1},
+                                     bulk))
             return rc;
         }
       }
@@ -585,13 +581,20 @@ extern "C" int llmc_chol_inv_upper(float* A, int64_t C, void* workspace, int64_t
         float* T = Y + k0 * n;
         float* Th = Yhi + k0 * n;
         float* Tl = Ylo + k0 * n;
-        if (int rc = tf32x3_update(Xh, Xl, 0, n, Th, Tl, 1, n, T, n, nb, k0, nb, 1, 0, 0, 0, Th, Tl, si))
+        if (int rc = tf32x3_update({.Ahi = Xh, .Alo = Xl, .lda = n,
+                                    .Bhi = Th, .Blo = Tl, .b_mn = 1, .ldb = n,
+                                    .C = T, .ldc = n, .M = nb, .N = k0, .K = nb, .mode = 1,
+                                    .Chi = Th, .Clo = Tl},
+                                   si))
           return rc;
       }
       if (m > 0 && r0 < sp1) {
-        if (int rc = tf32x3_update_ex(Lhi + r0 * n + k0, Llo + r0 * n + k0, 0, n, Yhi + k0 * n,
-                                      Ylo + k0 * n, 1, n, Y + r0 * n, n, sp1 - r0, r0, nb, 0, 0, 0, 0,
-                                      Yhi + r0 * n, Ylo + r0 * n, NB, 0, si))
+        if (int rc = tf32x3_update({.Ahi = Lhi + r0 * n + k0, .Alo = Llo + r0 * n + k0, .lda = n,
+                                    .Bhi = Yhi + k0 * n, .Blo = Ylo + k0 * n, .b_mn = 1, .ldb = n,
+                                    .C = Y + r0 * n, .ldc = n, .M = sp1 - r0, .N = r0, .K = nb,
+                                    .mode = 0, .Chi = Yhi + r0 * n, .Clo = Ylo + r0 * n,
+                                    .split_rows = NB, .split_cols = 0},
+                                   si))
           return rc;
       } else if (m > 0) {
         // T'[sp1:, 0:sp1] -= L[sp1:, sp0:sp1] Y[sp0:sp1, 0:sp1]: the next super-panel's rows on the
@@ -600,16 +603,21 @@ extern "C" int llmc_chol_inv_upper(float* A, int64_t C, void* workspace, int64_t
         const int kk = static_cast<int>(sp1 - sp0);
         const int64_t ra = (sp1 + spw < n) ? sp1 + spw : n;
         if (sidx > 0) LLMC_CHECK_CUDA(cudaStreamWaitEvent(si, evIB[sidx - 1], 0));
-        if (int rc = tf32x3_update_ex(Lhi + sp1 * n + sp0, Llo + sp1 * n + sp0, 0, n, Yhi + sp0 * n,
-                                      Ylo + sp0 * n, 1, n, Y + sp1 * n, n, ra - sp1, sp1, kk, 0, 0, 0, 0,
-                                      Yhi + sp1 * n, Ylo + sp1 * n, NB, 0, si))
+        if (int rc = tf32x3_update({.Ahi = Lhi + sp1 * n + sp0, .Alo = Llo + sp1 * n + sp0, .lda = n,
+                                    .Bhi = Yhi + sp0 * n, .Blo = Ylo + sp0 * n, .b_mn = 1, .ldb = n,
+                                    .C = Y + sp1 * n, .ldc = n, .M = ra - sp1, .N = sp1, .K = kk,
+                                    .mode = 0, .Chi = Yhi + sp1 * n, .Clo = Ylo + sp1 * n,
+                                    .split_rows = NB, .split_cols = 0},
+                                   si))
           return rc;
         LLMC_CHECK_CUDA(cudaEventRecord(evI[sidx], si));
         LLMC_CHECK_CUDA(cudaStreamWaitEvent(s3, evI[sidx], 0));
         if (ra < n) {
-          if (int rc = tf32x3_update_grid(Lhi + ra * n + sp0, Llo + ra * n + sp0, 0, n, Yhi + sp0 * n,
-                                          Ylo + sp0 * n, 1, n, Y + ra * n, n, n - ra, sp1, kk, 0, 0, 0, 0,
-                                          nullptr, nullptr, 0, 0, 1, s3))
+          if (int rc = tf32x3_update({.Ahi = Lhi + ra * n + sp0, .Alo = Llo + ra * n + sp0, .lda = n,
+                                      .Bhi = Yhi + sp0 * n, .Blo = Ylo + sp0 * n, .b_mn = 1, .ldb = n,
+                                      .C = Y + ra * n, .ldc = n, .M = n - ra, .N = sp1, .K = kk,
+                                      .mode = 0, .one_tile_per_cta = 1},
+                                     s3))
             return rc;
         }
         LLMC_CHECK_CUDA(cudaEventRecord(evIB[sidx], s3));
@@ -655,7 +663,10 @@ extern "C" int llmc_chol_inv_upper(float* A, int64_t C, void* workspace, int64_t
       if (kb == 0)
         if (int rc = split_tf32(P, m, nb, n, Ph, Pl, n, st)) return rc;
       // P <- P * L_kk^-T : out[i][j] = sum_k P[i][k] * Dk[j][k]   (both K-major), + split
-      if (int rc = tf32x3_update(Ph, Pl, 0, n, Xh, Xl, 0, ldx, P, n, m, nb, nb, 1, 0, 0, 0, Ph, Pl, st))
+      if (int rc = tf32x3_update({.Ahi = Ph, .Alo = Pl, .lda = n, .Bhi = Xh, .Blo = Xl, .ldb = ldx,
+                                  .C = P, .ldc = n, .M = m, .N = nb, .K = nb, .mode = 1,
+                                  .Chi = Ph, .Clo = Pl},
+                                 st))
         return rc;
     }
     LLMC_CHECK_CUDA(cudaEventRecord(ev[kb], st));          // L panel kb, D_kb and Y_kk are final
@@ -667,16 +678,22 @@ extern "C" int llmc_chol_inv_upper(float* A, int64_t C, void* workspace, int64_t
     const int64_t sp1 = (sp0 + spw < n) ? sp0 + spw : n;
     if (m > 0 && r0 < sp1) {
       // G[r0:, r0:sp1] -= P P[r0:sp1]^T  (lower tiles only)
-      if (int rc = tf32x3_update_ex(Ph, Pl, 0, n, Ph, Pl, 0, n, G + r0 * n + r0, n, m, sp1 - r0, nb, 0,
-                                    1, 0, 0, Lhi + r0 * n + r0, Llo + r0 * n + r0, 0, NB, st))
+      if (int rc = tf32x3_update({.Ahi = Ph, .Alo = Pl, .lda = n, .Bhi = Ph, .Blo = Pl, .ldb = n,
+                                  .C = G + r0 * n + r0, .ldc = n, .M = m, .N = sp1 - r0, .K = nb,
+                                  .mode = 0, .Chi = Lhi + r0 * n + r0, .Clo = Llo + r0 * n + r0,
+                                  .split_rows = 0, .split_cols = NB, .tri = 1},
+                                 st))
         return rc;
     } else if (m > 0) {
       // G[sp1:, sp1:] -= L[sp1:, sp0:sp1] L[sp1:, sp0:sp1]^T
       const float* Ah = Lhi + sp1 * n + sp0;
       const float* Al = Llo + sp1 * n + sp0;
-      if (int rc = tf32x3_update_ex(Ah, Al, 0, n, Ah, Al, 0, n, G + sp1 * n + sp1, n, n - sp1, n - sp1,
-                                    static_cast<int>(sp1 - sp0), 0, 1, 0, 0, Lhi + sp1 * n + sp1,
-                                    Llo + sp1 * n + sp1, 0, NB, st))
+      if (int rc = tf32x3_update({.Ahi = Ah, .Alo = Al, .lda = n, .Bhi = Ah, .Blo = Al, .ldb = n,
+                                  .C = G + sp1 * n + sp1, .ldc = n, .M = n - sp1, .N = n - sp1,
+                                  .K = static_cast<int>(sp1 - sp0), .mode = 0,
+                                  .Chi = Lhi + sp1 * n + sp1, .Clo = Llo + sp1 * n + sp1,
+                                  .split_rows = 0, .split_cols = NB, .tri = 1},
+                                 st))
         return rc;
     }
 
@@ -689,21 +706,31 @@ extern "C" int llmc_chol_inv_upper(float* A, int64_t C, void* workspace, int64_t
       float* Th = Yhi + k0 * n;
       float* Tl = Ylo + k0 * n;
       // Y[k rows, 0:k0] = D_k (K-major: D[m][kk]) * T' (MN-major: element (col, kk) at T[kk*n + col])
-      if (int rc = tf32x3_update(Xh, Xl, 0, ldx, Th, Tl, 1, n, T, n, nb, k0, nb, 1, 0, 0, 0, Th, Tl, s2))
+      if (int rc = tf32x3_update({.Ahi = Xh, .Alo = Xl, .lda = ldx,
+                                  .Bhi = Th, .Blo = Tl, .b_mn = 1, .ldb = n,
+                                  .C = T, .ldc = n, .M = nb, .N = k0, .K = nb, .mode = 1,
+                                  .Chi = Th, .Clo = Tl},
+                                 s2))
         return rc;
     }
     if (m > 0 && r0 < sp1) {
       // T'[r0:sp1, 0:r0] -= L[r0:sp1, kblock] * Y[k rows, 0:r0]; emits the split of the next T' rows
-      if (int rc = tf32x3_update_ex(Lhi + r0 * n + k0, Llo + r0 * n + k0, 0, n, Yhi + k0 * n,
-                                    Ylo + k0 * n, 1, n, Y + r0 * n, n, sp1 - r0, r0, nb, 0, 0, 0, 0,
-                                    Yhi + r0 * n, Ylo + r0 * n, NB, 0, s2))
+      if (int rc = tf32x3_update({.Ahi = Lhi + r0 * n + k0, .Alo = Llo + r0 * n + k0, .lda = n,
+                                  .Bhi = Yhi + k0 * n, .Blo = Ylo + k0 * n, .b_mn = 1, .ldb = n,
+                                  .C = Y + r0 * n, .ldc = n, .M = sp1 - r0, .N = r0, .K = nb,
+                                  .mode = 0, .Chi = Yhi + r0 * n, .Clo = Ylo + r0 * n,
+                                  .split_rows = NB, .split_cols = 0},
+                                 s2))
         return rc;
     } else if (m > 0) {
       // T'[sp1:, 0:sp1] -= L[sp1:, sp0:sp1] * Y[sp0:sp1, 0:sp1]
-      if (int rc = tf32x3_update_ex(Lhi + sp1 * n + sp0, Llo + sp1 * n + sp0, 0, n, Yhi + sp0 * n,
-                                    Ylo + sp0 * n, 1, n, Y + sp1 * n, n, n - sp1, sp1,
-                                    static_cast<int>(sp1 - sp0), 0, 0, 0, 0, Yhi + sp1 * n,
-                                    Ylo + sp1 * n, NB, 0, s2))
+      if (int rc = tf32x3_update({.Ahi = Lhi + sp1 * n + sp0, .Alo = Llo + sp1 * n + sp0, .lda = n,
+                                  .Bhi = Yhi + sp0 * n, .Blo = Ylo + sp0 * n, .b_mn = 1, .ldb = n,
+                                  .C = Y + sp1 * n, .ldc = n, .M = n - sp1, .N = sp1,
+                                  .K = static_cast<int>(sp1 - sp0), .mode = 0,
+                                  .Chi = Yhi + sp1 * n, .Clo = Ylo + sp1 * n,
+                                  .split_rows = NB, .split_cols = 0},
+                                 s2))
         return rc;
     }
   }

@@ -4,7 +4,9 @@
 //   warp 0     TMA producer  (cp.async.bulk.tensor -> 128B-swizzled smem ring, mbarrier tx)
 //   warp 1     MMA issuer    (one elected thread, tcgen05.mma kind::f16, fp32 accum in TMEM)
 //   warps 2-5  epilogue      (tcgen05.ld TMEM -> registers -> global), double-buffered TMEM
-// Tile 128(M) x 256(N) x 64(K), 4-stage ring (48 KB / stage), 2 x 256 TMEM columns.
+// Tile 128(M) x 256(N) x 64(K), 4-stage ring (48 KB / stage), 2 x 256 TMEM columns.  The
+// scaffolding (TMEM setup, rings, rasterisation, epilogue stores, launch) comes from tc.cuh; this
+// file also defines the tensor-map encoder declared there.
 //
 //  * GEMM  (llmc_gemm_bf16):  Y[M,N] = X[M,K] . W[N,K]^T (+bias) — both operands K-major.
 //      Replaces F.linear in FakeQuantLinear / EffcientFakeQuantLinear.forward
@@ -53,17 +55,8 @@ template <bool kSyrk>
 __device__ __forceinline__ Unit decode_unit(const GemmParams& p, int u) {
   Unit t;
   if constexpr (!kSyrk) {
-    // Grouped rasterisation: weights are swept in groups of `gn` n-tiles (<= ~32 MB, L2 resident),
-    // all m-tiles per group, n fastest inside the group.  Activations are re-read N/(256*gn)
-    // times from HBM, weights once; n-fastest over a 14336-row weight would instead stream the
-    // whole 117 MB weight through L2 once per 148-tile wave.
-    const int m_tiles = p.num_tiles / p.n_tiles_n;
-    const int per_group = p.gn * m_tiles;
-    const int g = u / per_group;
-    const int rem = u - g * per_group;
-    const int gsz = min(p.gn, p.n_tiles_n - g * p.gn);
-    t.m_blk = rem / gsz;
-    t.n_blk = g * p.gn + (rem - t.m_blk * gsz);
+    // (a 14336-row weight is 117 MB: n-fastest order would stream all of it per 148-tile wave)
+    grouped_tile(u, p.num_tiles / p.n_tiles_n, p.n_tiles_n, p.gn, t.m_blk, t.n_blk);
     t.kb0 = 0;
     t.kb1 = p.kb_total;
     t.split = 0;
@@ -102,9 +95,7 @@ template <bool kSyrk, bool kBf16>
 __global__ void __launch_bounds__(kThreads, 1)
 umma_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const GemmParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
-                                             ~static_cast<uintptr_t>(1023));
+  uint8_t* smem = smem_align1024();
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + kStages * kStageBytes);
   uint64_t* empty_bar = full_bar + kStages;
   uint64_t* tmem_full = empty_bar + kStages;
@@ -127,59 +118,51 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     }
     fence_barrier_init();
   }
-  if (warp == 1) tmem_alloc(tmem_ptr, kTmemCols);
-  tcgen05_fence_before();
-  __syncthreads();
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
+  const uint32_t tmem_base = tmem_setup(warp, tmem_ptr, kTmemCols);
 
   if (warp == 0) {
     // ===================== TMA producer =====================
     if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
+      Ring<kStages> s;
       for (int u = blockIdx.x; u < p.num_units; u += gridDim.x) {
         const Unit t = decode_unit<kSyrk>(p, u);
         for (int kb = t.kb0; kb < t.kb1; ++kb) {
-          mbar_wait(&empty_bar[stage], phase ^ 1);
-          uint8_t* a_dst = smem + stage * kStageBytes;
+          mbar_wait(&empty_bar[s.idx], s.phase ^ 1);
+          uint8_t* a_dst = smem + s.idx * kStageBytes;
           uint8_t* b_dst = a_dst + kABytes;
-          mbar_expect_tx(&full_bar[stage], kStageBytes);
+          uint64_t* bar = &full_bar[s.idx];
+          mbar_expect_tx(bar, kStageBytes);
           if constexpr (!kSyrk) {
-            tma_load_2d(a_dst, &tmA, &full_bar[stage], kb * BK, t.m_blk * BM);
-            tma_load_2d(b_dst, &tmB, &full_bar[stage], kb * BK, t.n_blk * BN);
+            tma_load_2d(a_dst, &tmA, bar, kb * BK, t.m_blk * BM);
+            tma_load_2d(b_dst, &tmB, bar, kb * BK, t.n_blk * BN);
           } else {
             // X[T, C]: coordinate 0 = channel, coordinate 1 = token; box = 64 ch x 64 tok
 #pragma unroll
             for (int i = 0; i < BM / 64; ++i)
-              tma_load_2d(a_dst + i * kBoxBytes, &tmA, &full_bar[stage], t.m_blk * BM + i * 64,
-                          kb * BK);
+              tma_load_2d(a_dst + i * kBoxBytes, &tmA, bar, t.m_blk * BM + i * 64, kb * BK);
 #pragma unroll
             for (int i = 0; i < BN / 64; ++i)
-              tma_load_2d(b_dst + i * kBoxBytes, &tmA, &full_bar[stage], t.n_blk * BN + i * 64,
-                          kb * BK);
+              tma_load_2d(b_dst + i * kBoxBytes, &tmA, bar, t.n_blk * BN + i * 64, kb * BK);
           }
-          if (++stage == kStages) { stage = 0; phase ^= 1; }
+          s.advance();
         }
       }
     }
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
-    constexpr uint32_t idesc = make_idesc_f16(kBf16 ? 1 : 0, kSyrk ? 1 : 0, kSyrk ? 1 : 0, BM, BN);
-    int stage = 0;
-    uint32_t phase = 0;
-    int as = 0;
-    uint32_t aphase = 0;
+    constexpr uint32_t idesc = make_idesc(kBf16, kBf16, kSyrk, kSyrk, BM, BN);
+    Ring<kStages> s;
+    Ring<2> acc;
     for (int u = blockIdx.x; u < p.num_units; u += gridDim.x) {
       const Unit t = decode_unit<kSyrk>(p, u);
-      mbar_wait(&tmem_empty[as], aphase ^ 1);
+      mbar_wait(&tmem_empty[acc.idx], acc.phase ^ 1);
       tcgen05_fence_after();
-      const uint32_t d_tmem = tmem_base + as * BN;
+      const uint32_t d_tmem = tmem_base + acc.idx * BN;
       for (int kb = t.kb0; kb < t.kb1; ++kb) {
-        mbar_wait(&full_bar[stage], phase);
+        mbar_wait(&full_bar[s.idx], s.phase);
         tcgen05_fence_after();
         if (lane == 0) {
-          const uint32_t a_addr = smem_u32(smem + stage * kStageBytes);
+          const uint32_t a_addr = smem_u32(smem + s.idx * kStageBytes);
           const uint32_t b_addr = a_addr + kABytes;
 #pragma unroll
           for (int k = 0; k < BK / 16; ++k) {
@@ -193,27 +176,25 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             }
             umma_f16(d_tmem, adesc, bdesc, idesc, (kb > t.kb0 || k > 0) ? 1u : 0u);
           }
-          umma_commit(&empty_bar[stage]);                    // frees the smem slot
-          if (kb == t.kb1 - 1) umma_commit(&tmem_full[as]);  // accumulator complete
+          umma_commit(&empty_bar[s.idx]);                         // frees the smem slot
+          if (kb == t.kb1 - 1) umma_commit(&tmem_full[acc.idx]);  // accumulator complete
         }
         __syncwarp();
-        if (++stage == kStages) { stage = 0; phase ^= 1; }
+        s.advance();
       }
-      if (t.kb1 <= t.kb0 && lane == 0) umma_commit(&tmem_full[as]);  // empty K range (never)
-      as ^= 1;
-      if (as == 0) aphase ^= 1;
+      if (t.kb1 <= t.kb0 && lane == 0) umma_commit(&tmem_full[acc.idx]);  // empty K range (never)
+      acc.advance();
     }
   } else {
     // ===================== epilogue (warps 2..5) =====================
     const int q = warp & 3;                       // TMEM lane quarter this warp may access
-    int as = 0;
-    uint32_t aphase = 0;
+    Ring<2> acc;
     for (int u = blockIdx.x; u < p.num_units; u += gridDim.x) {
       const Unit t = decode_unit<kSyrk>(p, u);
-      mbar_wait(&tmem_full[as], aphase);
+      mbar_wait(&tmem_full[acc.idx], acc.phase);
       tcgen05_fence_after();
       const int64_t row = static_cast<int64_t>(t.m_blk) * BM + q * 32 + lane;
-      const uint32_t taddr0 = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + as * BN;
+      const uint32_t taddr0 = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc.idx * BN;
 #pragma unroll 1
       for (int c = 0; c < BN; c += 32) {
         uint32_t r[32];
@@ -232,50 +213,19 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
               for (int i = 0; i < 32 && col0 + i < p.N; ++i) o[i] = __uint_as_float(r[i]);
             }
           } else {
-            uint16_t* o = reinterpret_cast<uint16_t*>(p.out) + row * p.ld_out + col0;
-            const uint16_t* bs = reinterpret_cast<const uint16_t*>(p.bias);
-            const bool full = (col0 + 32 <= p.N) && ((p.ld_out & 7) == 0);
-            uint32_t pk[16];
-#pragma unroll
-            for (int i = 0; i < 32; i += 2) {
-              float v0 = __uint_as_float(r[i]), v1 = __uint_as_float(r[i + 1]);
-              if (bs != nullptr) {
-                // F.linear adds the bias in fp32 before the single rounding to the out dtype
-                if (col0 + i < p.N) v0 += kBf16 ? __uint_as_float(static_cast<uint32_t>(bs[col0 + i]) << 16)
-                                                : __half2float(__ushort_as_half(bs[col0 + i]));
-                if (col0 + i + 1 < p.N) v1 += kBf16 ? __uint_as_float(static_cast<uint32_t>(bs[col0 + i + 1]) << 16)
-                                                    : __half2float(__ushort_as_half(bs[col0 + i + 1]));
-              }
-              if constexpr (kBf16) {
-                __nv_bfloat162 h = __floats2bfloat162_rn(v0, v1);
-                pk[i >> 1] = *reinterpret_cast<uint32_t*>(&h);
-              } else {
-                __half2 h = __floats2half2_rn(v0, v1);
-                pk[i >> 1] = *reinterpret_cast<uint32_t*>(&h);
-              }
-            }
-            if (full) {
-#pragma unroll
-              for (int i = 0; i < 16; i += 4)
-                *reinterpret_cast<uint4*>(o + 2 * i) = make_uint4(pk[i], pk[i + 1], pk[i + 2], pk[i + 3]);
-            } else {
-              for (int i = 0; i < 32 && col0 + i < p.N; ++i)
-                o[i] = static_cast<uint16_t>((i & 1) ? (pk[i >> 1] >> 16) : (pk[i >> 1] & 0xffffu));
-            }
+            store_chunk_bias<kBf16>(reinterpret_cast<uint16_t*>(p.out) + row * p.ld_out + col0, r,
+                                    reinterpret_cast<const uint16_t*>(p.bias), col0, p.N,
+                                    (p.ld_out & 7) == 0);
           }
         }
       }
       tcgen05_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive(&tmem_empty[as]);
-      as ^= 1;
-      if (as == 0) aphase ^= 1;
+      if (lane == 0) mbar_arrive(&tmem_empty[acc.idx]);
+      acc.advance();
     }
   }
-
-  tcgen05_fence_before();
-  __syncthreads();
-  if (warp == 1) tmem_dealloc(tmem_base, kTmemCols);
+  tmem_teardown(warp, tmem_base, kTmemCols);
 }
 
 // ---- SYRK finalize: H = a*H + b*sum_s P_s on the upper triangle, mirrored -----------------------
@@ -337,86 +287,22 @@ static PFN_tmapEncodeTiled get_encode_fn() {
   return fn;
 }
 
-int encode_tmap_2d_b16(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
-                       uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols) {
+int encode_tmap_2d(CUtensorMap* out, const void* base, CUtensorMapDataType dtype,
+                   uint32_t elem_bytes, uint64_t rows, uint64_t cols, uint64_t ld_elems,
+                   uint32_t box_rows, uint32_t box_cols, CUtensorMapSwizzle swizzle) {
   PFN_tmapEncodeTiled fn = get_encode_fn();
   if (!fn) return LLMC_ECUDA;
   cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {ld_elems * 2};
+  cuuint64_t strides[1] = {ld_elems * elem_bytes};
   cuuint32_t box[2] = {box_cols, box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides,
-                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  CUresult r = fn(out, dtype, 2, const_cast<void*>(base), dims, strides, box, estr,
+                  CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
-    set_last_error("cuTensorMapEncodeTiled failed with CUresult %d (rows %llu cols %llu ld %llu)",
-                   (int)r, (unsigned long long)rows, (unsigned long long)cols,
-                   (unsigned long long)ld_elems);
-    return LLMC_ECUDA;
-  }
-  return LLMC_OK;
-}
-
-int encode_tmap_2d_u8(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
-                      uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols) {
-  PFN_tmapEncodeTiled fn = get_encode_fn();
-  if (!fn) return LLMC_ECUDA;
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {ld_elems};
-  cuuint32_t box[2] = {box_cols, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base), dims, strides,
-                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_last_error("cuTensorMapEncodeTiled(u8) failed with CUresult %d (rows %llu cols %llu ld %llu)",
-                   (int)r, (unsigned long long)rows, (unsigned long long)cols,
-                   (unsigned long long)ld_elems);
-    return LLMC_ECUDA;
-  }
-  return LLMC_OK;
-}
-
-int encode_tmap_2d_f32(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
-                       uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols, int atom32b) {
-  PFN_tmapEncodeTiled fn = get_encode_fn();
-  if (!fn) return LLMC_ECUDA;
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {ld_elems * 4};
-  cuuint32_t box[2] = {box_cols, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(base), dims, strides,
-                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  atom32b ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B,
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_last_error("cuTensorMapEncodeTiled(f32) failed with CUresult %d (rows %llu cols %llu ld %llu)",
-                   (int)r, (unsigned long long)rows, (unsigned long long)cols,
-                   (unsigned long long)ld_elems);
-    return LLMC_ECUDA;
-  }
-  return LLMC_OK;
-}
-
-// swizzle32: CU_TENSOR_MAP_SWIZZLE_32B (box_cols must be 8 = 32 bytes): the 16-byte half of a
-// 32-byte row is XORed with bit 2 of the row index, which makes one-row-per-thread 16-byte
-// shared-memory loads conflict free.
-int encode_tmap_2d_i32_noswizzle(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
-                                 uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols,
-                                 int swizzle32) {
-  PFN_tmapEncodeTiled fn = get_encode_fn();
-  if (!fn) return LLMC_ECUDA;
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {ld_elems * 4};
-  cuuint32_t box[2] = {box_cols, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, const_cast<void*>(base), dims, strides, box,
-                  estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  swizzle32 == 2 ? CU_TENSOR_MAP_SWIZZLE_64B
-                                 : (swizzle32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_NONE),
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_last_error("cuTensorMapEncodeTiled(i32) failed with CUresult %d", (int)r);
+    set_last_error("cuTensorMapEncodeTiled failed with CUresult %d (dtype %d rows %llu cols %llu "
+                   "ld %llu box %ux%u)", (int)r, (int)dtype, (unsigned long long)rows,
+                   (unsigned long long)cols, (unsigned long long)ld_elems, box_rows, box_cols);
     return LLMC_ECUDA;
   }
   return LLMC_OK;
@@ -425,14 +311,8 @@ int encode_tmap_2d_i32_noswizzle(CUtensorMap* out, const void* base, uint64_t ro
 template <bool kSyrk, bool kBf16>
 static int launch_umma(const CUtensorMap& tmA, const CUtensorMap& tmB, const GemmParams& p,
                        cudaStream_t st) {
-  auto kern = umma_gemm_kernel<kSyrk, kBf16>;
-  LLMC_ONCE_PER_DEVICE({
-    LLMC_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  });
-  int grid = p.num_units < kNumSMs ? p.num_units : kNumSMs;
-  kern<<<grid, kThreads, kSmemBytes, st>>>(tmA, tmB, p);
-  LLMC_CHECK_LAUNCH();
-  return LLMC_OK;
+  const int grid = p.num_units < kNumSMs ? p.num_units : kNumSMs;
+  return launch_tc<umma_gemm_kernel<kSyrk, kBf16>>(grid, kThreads, kSmemBytes, st, tmA, tmB, p);
 }
 
 struct SyrkPlan {
@@ -481,8 +361,12 @@ extern "C" int llmc_gemm_bf16(const void* x, const void* w, const void* bias, vo
     return LLMC_EALIGN;
   }
   CUtensorMap tmA, tmB;
-  if (int rc = encode_tmap_2d_b16(&tmA, x, M, K, K, BM, BK)) return rc;
-  if (int rc = encode_tmap_2d_b16(&tmB, w, N, K, K, BN, BK)) return rc;
+  if (int rc = encode_tmap_2d(&tmA, x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, M, K, K, BM, BK,
+                              CU_TENSOR_MAP_SWIZZLE_128B))
+    return rc;
+  if (int rc = encode_tmap_2d(&tmB, w, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, N, K, K, BN, BK,
+                              CU_TENSOR_MAP_SWIZZLE_128B))
+    return rc;
   GemmParams p{};
   p.M = M; p.N = N; p.K = K;
   p.out = y; p.bias = bias; p.ld_out = N;
@@ -494,13 +378,7 @@ extern "C" int llmc_gemm_bf16(const void* x, const void* w, const void* bias, vo
   p.splits = 1;
   p.kb_total = static_cast<int>((K + BK - 1) / BK);
   p.kb_per_split = p.kb_total;
-  {
-    const int64_t tile_bytes = static_cast<int64_t>(BN) * K * 2;      // one n-tile of weights
-    int64_t gn = (32ll << 20) / (tile_bytes > 0 ? tile_bytes : 1);
-    if (gn < 1) gn = 1;
-    if (gn > p.n_tiles_n) gn = p.n_tiles_n;
-    p.gn = static_cast<int>(gn);
-  }
+  p.gn = raster_group_n(static_cast<int64_t>(BN) * K * 2, p.n_tiles_n);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   return dtype == LLMC_BF16 ? launch_umma<false, true>(tmA, tmB, p, st)
                             : launch_umma<false, false>(tmA, tmB, p, st);
@@ -526,7 +404,9 @@ extern "C" int llmc_syrk_accum(const void* x, int64_t T, int64_t C, int dtype, f
                  "syrk: workspace too small (%lld < %lld)", (long long)workspace_bytes,
                  (long long)(static_cast<int64_t>(s.splits) * C * C * 4));
   CUtensorMap tmX;
-  if (int rc = encode_tmap_2d_b16(&tmX, x, T, C, C, 64, 64)) return rc;
+  if (int rc = encode_tmap_2d(&tmX, x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, T, C, C, 64, 64,
+                              CU_TENSOR_MAP_SWIZZLE_128B))
+    return rc;
   GemmParams p{};
   p.M = C; p.N = C; p.K = T;
   p.out = workspace; p.bias = nullptr; p.ld_out = C;

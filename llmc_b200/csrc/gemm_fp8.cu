@@ -22,6 +22,7 @@
 //      `n // 128` indexing assumes.  Ragged M and N: TMA zero-fill and masked stores.
 //      Optional bias (bf16 output only) follows block_wise_fp8_forward_func: the fp32 result is
 //      rounded to bf16 and then `y += bias` rounds bf16(float(y) + float(bias)) once more.
+//      The scaffolding (TMEM setup, rings, rasterisation, 16-bit stores, launch) comes from tc.cuh.
 #include "tc.cuh"
 
 namespace llmc {
@@ -51,16 +52,6 @@ struct Params {
   int gn;                   // rasterisation group (n-tiles)
 };
 
-__device__ __forceinline__ void decode_tile(const Params& p, int u, int& m_blk, int& n_blk) {
-  // groups of `gn` n-tiles (weights L2-resident), all m-tiles per group, n fastest inside
-  const int per_group = p.gn * p.m_tiles;
-  const int g = u / per_group;
-  const int rem = u - g * per_group;
-  const int gsz = min(p.gn, p.n_tiles_n - g * p.gn);
-  m_blk = rem / gsz;
-  n_blk = g * p.gn + (rem - m_blk * gsz);
-}
-
 __device__ __forceinline__ float bias_at(const Params& p, int64_t col) {
   if (p.bias_dtype == LLMC_F32) return reinterpret_cast<const float*>(p.bias)[col];
   return __uint_as_float(static_cast<uint32_t>(reinterpret_cast<const uint16_t*>(p.bias)[col]) << 16);
@@ -86,40 +77,28 @@ __device__ __forceinline__ void store_chunk(const Params& p, int64_t row, int64_
   if (p.out_dtype == LLMC_BF16) {
 #pragma unroll
     for (int i = 0; i < 32; i += 2) {
-      __nv_bfloat162 h = __floats2bfloat162_rn(v[i], v[i + 1]);
+      pk[i >> 1] = pack2<true>(v[i], v[i + 1]);
       if (p.bias != nullptr) {
         // `y += bias`: bf16 y and fp32 / bf16 bias meet in fp32, one more rounding to bf16
         const float b0 = i < n_valid ? bias_at(p, col0 + i) : 0.f;
         const float b1 = i + 1 < n_valid ? bias_at(p, col0 + i + 1) : 0.f;
-        h = __floats2bfloat162_rn(__low2float(h) + b0, __high2float(h) + b1);
+        pk[i >> 1] = pack2<true>(__uint_as_float(pk[i >> 1] << 16) + b0,
+                                 __uint_as_float(pk[i >> 1] & 0xffff0000u) + b1);
       }
-      pk[i >> 1] = *reinterpret_cast<uint32_t*>(&h);
     }
   } else {
 #pragma unroll
-    for (int i = 0; i < 32; i += 2) {
-      __half2 h = __floats2half2_rn(v[i], v[i + 1]);
-      pk[i >> 1] = *reinterpret_cast<uint32_t*>(&h);
-    }
+    for (int i = 0; i < 32; i += 2) pk[i >> 1] = pack2<false>(v[i], v[i + 1]);
   }
-  uint16_t* o = reinterpret_cast<uint16_t*>(p.out) + row * p.N + col0;
-  if (n_valid >= 32 && (p.N & 7) == 0) {
-#pragma unroll
-    for (int i = 0; i < 16; i += 4)
-      *reinterpret_cast<uint4*>(o + 2 * i) = make_uint4(pk[i], pk[i + 1], pk[i + 2], pk[i + 3]);
-  } else {
-#pragma unroll
-    for (int i = 0; i < 32; ++i)
-      if (i < n_valid) o[i] = static_cast<uint16_t>((i & 1) ? (pk[i >> 1] >> 16) : (pk[i >> 1] & 0xffffu));
-  }
+  // columns counted from the chunk's start: the first n_valid are inside the row
+  store_row32_b16(reinterpret_cast<uint16_t*>(p.out) + row * p.N + col0, pk,
+                  n_valid >= 32 && (p.N & 7) == 0, 0, n_valid);
 }
 
 __global__ void __launch_bounds__(kThreads, 1)
 fp8_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                 const Params p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
-                                             ~static_cast<uintptr_t>(1023));
+  uint8_t* smem = smem_align1024();
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + kStages * kStageBytes);
   uint64_t* empty_bar = full_bar + kStages;
   uint64_t* tmem_full = empty_bar + kStages;
@@ -142,64 +121,58 @@ fp8_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     }
     fence_barrier_init();
   }
-  if (warp == 1) tmem_alloc(tmem_ptr, kTmemCols);
-  tcgen05_fence_before();
-  __syncthreads();
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
+  const uint32_t tmem_base = tmem_setup(warp, tmem_ptr, kTmemCols);
 
   if (warp == 0) {
     // ===================== TMA producer =====================
     if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
+      Ring<kStages> s;
       for (int u = blockIdx.x; u < p.num_tiles; u += gridDim.x) {
         int m_blk, n_blk;
-        decode_tile(p, u, m_blk, n_blk);
+        grouped_tile(u, p.m_tiles, p.n_tiles_n, p.gn, m_blk, n_blk);
         for (int kb = 0; kb < p.kb_total; ++kb) {
-          mbar_wait(&empty_bar[stage], phase ^ 1);
-          uint8_t* a_dst = smem + stage * kStageBytes;
-          mbar_expect_tx(&full_bar[stage], kStageBytes);
-          tma_load_2d(a_dst, &tmA, &full_bar[stage], kb * BK, m_blk * BM);
-          tma_load_2d(a_dst + kTileBytes, &tmB, &full_bar[stage], kb * BK, n_blk * BN);
-          if (++stage == kStages) { stage = 0; phase ^= 1; }
+          mbar_wait(&empty_bar[s.idx], s.phase ^ 1);
+          uint8_t* a_dst = smem + s.idx * kStageBytes;
+          mbar_expect_tx(&full_bar[s.idx], kStageBytes);
+          tma_load_2d(a_dst, &tmA, &full_bar[s.idx], kb * BK, m_blk * BM);
+          tma_load_2d(a_dst + kTileBytes, &tmB, &full_bar[s.idx], kb * BK, n_blk * BN);
+          s.advance();
         }
       }
     }
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
-    constexpr uint32_t idesc = make_idesc_e4m3(BM, BN);
-    int stage = 0, slot = 0;
-    uint32_t phase = 0, sphase = 0;
+    constexpr uint32_t idesc = make_idesc(0, 0, 0, 0, BM, BN);     // e4m3 x e4m3, both K-major
+    Ring<kStages> s;
+    Ring<kSlots> slot;
     for (int u = blockIdx.x; u < p.num_tiles; u += gridDim.x) {
       for (int kb = 0; kb < p.kb_total; ++kb) {
-        mbar_wait(&tmem_empty[slot], sphase ^ 1);
-        mbar_wait(&full_bar[stage], phase);
+        mbar_wait(&tmem_empty[slot.idx], slot.phase ^ 1);
+        mbar_wait(&full_bar[s.idx], s.phase);
         tcgen05_fence_after();
         if (lane == 0) {
-          const uint32_t a_addr = smem_u32(smem + stage * kStageBytes);
+          const uint32_t a_addr = smem_u32(smem + s.idx * kStageBytes);
           const uint32_t b_addr = a_addr + kTileBytes;
-          const uint32_t d_tmem = tmem_base + slot * BN;
+          const uint32_t d_tmem = tmem_base + slot.idx * BN;
 #pragma unroll
           for (int k = 0; k < BK / 32; ++k)
             umma_f8f6f4(d_tmem, make_smem_desc(a_addr + k * 32, 16, 1024),
                         make_smem_desc(b_addr + k * 32, 16, 1024), idesc, k > 0 ? 1u : 0u);
-          umma_commit(&empty_bar[stage]);     // frees the smem slot
-          umma_commit(&tmem_full[slot]);      // this K-block's partial product is ready
+          umma_commit(&empty_bar[s.idx]);     // frees the smem slot
+          umma_commit(&tmem_full[slot.idx]);  // this K-block's partial product is ready
         }
         __syncwarp();
-        if (++stage == kStages) { stage = 0; phase ^= 1; }
-        if (++slot == kSlots) { slot = 0; sphase ^= 1; }
+        s.advance();
+        slot.advance();
       }
     }
   } else {
     // ===================== promotion + epilogue (warps 2..5) =====================
     const int q = warp & 3;                       // TMEM lane quarter this warp may access
-    int slot = 0;
-    uint32_t sphase = 0;
+    Ring<kSlots> slot;
     for (int u = blockIdx.x; u < p.num_tiles; u += gridDim.x) {
       int m_blk, n_blk;
-      decode_tile(p, u, m_blk, n_blk);
+      grouped_tile(u, p.m_tiles, p.n_tiles_n, p.gn, m_blk, n_blk);
       const int64_t row = static_cast<int64_t>(m_blk) * BM + q * 32 + lane;
       const bool row_ok = row < p.M;
       const float* as_row = p.a_s + (row_ok ? row : 0) * p.kb_total;
@@ -214,9 +187,9 @@ fp8_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         const int kn = kb + 1 < p.kb_total ? kb + 1 : kb;
         const float sa_next = row_ok ? __ldg(as_row + kn) : 0.f;
         const float sb_next = __ldg(bs_row + kn);
-        mbar_wait(&tmem_full[slot], sphase);
+        mbar_wait(&tmem_full[slot.idx], slot.phase);
         tcgen05_fence_after();
-        const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + slot * BN;
+        const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + slot.idx * BN;
 #pragma unroll
         for (int c = 0; c < BN; c += 32) {
           uint32_t r[32];
@@ -226,7 +199,7 @@ fp8_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             // the slot has been read out: hand it back before the last promotion
             tcgen05_fence_before();
             __syncwarp();
-            if (lane == 0) mbar_arrive(&tmem_empty[slot]);
+            if (lane == 0) mbar_arrive(&tmem_empty[slot.idx]);
           }
 #pragma unroll
           for (int i = 0; i < 32; i += 2)
@@ -235,7 +208,7 @@ fp8_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         }
         sa = sa_next;
         sb = sb_next;
-        if (++slot == kSlots) { slot = 0; sphase ^= 1; }
+        slot.advance();
       }
       const int64_t colt = static_cast<int64_t>(n_blk) * BN;
       if (row_ok) {
@@ -246,9 +219,7 @@ fp8_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     }
   }
 
-  tcgen05_fence_before();
-  __syncthreads();
-  if (warp == 1) tmem_dealloc(tmem_base, kTmemCols);
+  tmem_teardown(warp, tmem_base, kTmemCols);
 }
 
 // ---- act_quant ------------------------------------------------------------------------------
@@ -355,8 +326,12 @@ extern "C" int llmc_fp8_gemm(const void* a, const float* a_s, const void* b, con
     return LLMC_EALIGN;
   }
   CUtensorMap tmA, tmB;
-  if (int rc = encode_tmap_2d_u8(&tmA, a, M, K, K, BM, BK)) return rc;
-  if (int rc = encode_tmap_2d_u8(&tmB, b, N, K, K, BN, BK)) return rc;
+  if (int rc = encode_tmap_2d(&tmA, a, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, M, K, K, BM, BK,
+                              CU_TENSOR_MAP_SWIZZLE_128B))
+    return rc;
+  if (int rc = encode_tmap_2d(&tmB, b, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, N, K, K, BN, BK,
+                              CU_TENSOR_MAP_SWIZZLE_128B))
+    return rc;
   Params p{};
   p.M = M; p.N = N; p.K = K;
   p.a_s = a_s; p.b_s = b_s; p.out = c; p.bias = bias;
@@ -367,19 +342,8 @@ extern "C" int llmc_fp8_gemm(const void* a, const float* a_s, const void* b, con
   LLMC_CHECK_ARG(mt * p.n_tiles_n < (1ll << 31), "fp8_gemm: too many tiles");
   p.m_tiles = static_cast<int>(mt);
   p.num_tiles = static_cast<int>(mt * p.n_tiles_n);
-  {
-    int64_t gn = (32ll << 20) / (static_cast<int64_t>(BN) * K);   // ~32 MB of weights per group
-    if (gn < 1) gn = 1;
-    if (gn > p.n_tiles_n) gn = p.n_tiles_n;
-    p.gn = static_cast<int>(gn);
-  }
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  LLMC_ONCE_PER_DEVICE({
-    LLMC_CHECK_CUDA(cudaFuncSetAttribute(fp8_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         kSmemBytes));
-  });
+  p.gn = raster_group_n(static_cast<int64_t>(BN) * K, p.n_tiles_n);
   const int grid = p.num_tiles < kNumSMs ? p.num_tiles : kNumSMs;
-  fp8_gemm_kernel<<<grid, kThreads, kSmemBytes, st>>>(tmA, tmB, p);
-  LLMC_CHECK_LAUNCH();
-  return LLMC_OK;
+  return launch_tc<fp8_gemm_kernel>(grid, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream),
+                                    tmA, tmB, p);
 }

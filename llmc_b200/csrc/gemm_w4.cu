@@ -13,12 +13,15 @@
 //   ring L (4 x 24 KB): X tile [128 x 64] bf16 (swizzle 128B) + packed W tile [256 x 8] int32
 //   ring B (3 x 32 KB): the dequantised, 128B-swizzled UMMA B tile
 //   warp 0       TMA into ring L
-//   warps 6..13  dequant (one weight row per thread): nibble -> fp32 via the 2^23 magic constant,
+//   warps 6..13  dequant, two groups of four warps on alternate K steps (two weight rows per
+//                thread): nibble -> fp32 via the 2^23 magic constant,
 //                (q - z) * s in fp32, round to bf16/fp16, 16-byte stores into ring B,
 //                fence.proxy.async; the group's scale/zero for the NEXT step is prefetched
 //   warp 1       MMA issuer (tcgen05.mma kind::f16, 128 x 256 x 16, fp32 accumulators in TMEM);
 //                its commit frees the ring-L stage (X consumed) and the ring-B stage
-//   warps 2..5   epilogue (tcgen05.ld -> bias -> bf16/fp16 -> global), double-buffered TMEM
+//   warps 2..5   epilogue (tcgen05.ld -> bias -> bf16/fp16 -> global, the store of gemm.cu),
+//                double-buffered TMEM
+// The scaffolding (TMEM setup, rings, rasterisation, epilogue stores, launch) comes from tc.cuh.
 // Weight layout: LLMC_OUT_PACK_VLLM of UNSIGNED codes — 8 nibbles per int32 along K, nibble i =
 // element 8*w + i; scales / zeros fp32 [N, K/group] (zeros NULL => 2^(bit-1), the symmetric
 // +8 offset of module_utils.py:842-844).
@@ -33,22 +36,23 @@ using namespace tc;
 namespace w4 {
 
 constexpr int BM = 128, BN = 256, BK = 64;
-// ring B (dequantised W tile) depth and dequant warps are template parameters now: NG groups of
-// four warps take every NG-th K step (see the kernel), ring B is max(3, NG) deep
+// Two groups of four dequant warps take alternate K steps (see the kernel).  (A four-group
+// variant was tried in round 2 on the theory that the per-thread unpack chain, not issue
+// bandwidth, limits the kernel: it was slower, 728 vs 871 TFLOP/s, and was removed.)
+constexpr int NG = 2;
+constexpr int kThreads = (6 + 4 * NG) * 32;
+constexpr int kBStages = 3;                    // ring B (dequantised W tile)
 constexpr int kABytes = BM * BK * 2;          // 16 KB
 constexpr int kBBytes = BN * BK * 2;          // 32 KB dequantised
+constexpr int kTmemCols = 512;
 // per weight width: INT4 -> 8 KB packed tile, 4-deep ring L; INT8 -> 16 KB packed tile, 3-deep
-template <int kBits, int NG> struct Cfg {
+template <int kBits> struct Cfg {
   static constexpr int kPBytes = BN * BK * kBits / 8;
   static constexpr int kLBytes = kABytes + kPBytes;
-  static constexpr int kBStages = NG > 3 ? NG : 3;
-  static constexpr int kLStages = (kBits == 4 && NG <= 2) ? 4 : 3;
+  static constexpr int kLStages = kBits == 4 ? 4 : 3;
   static constexpr int kSmemBytes = kLStages * kLBytes + kBStages * kBBytes + 1024 + 256;
   static constexpr int kWordsPerRow = BK * kBits / 32;      // int32 per row of the packed tile
-  static constexpr int kDequantWarps = 4 * NG;
-  static constexpr int kThreads = (6 + kDequantWarps) * 32;
 };
-constexpr int kTmemCols = 512;
 
 struct Params {
   int64_t M, N, K;
@@ -65,24 +69,7 @@ struct Params {
 };
 
 __device__ __forceinline__ void decode(const Params& p, int u, int& m_blk, int& n_blk) {
-  const int m_tiles = p.num_units / p.n_tiles_n;
-  const int per_group = p.gn * m_tiles;
-  const int g = u / per_group;
-  const int rem = u - g * per_group;
-  const int gsz = min(p.gn, p.n_tiles_n - g * p.gn);
-  m_blk = rem / gsz;
-  n_blk = g * p.gn + (rem - m_blk * gsz);
-}
-
-template <bool kBf16>
-__device__ __forceinline__ uint32_t pack2(float a, float b) {
-  if constexpr (kBf16) {
-    __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-    return *reinterpret_cast<uint32_t*>(&h);
-  } else {
-    __half2 h = __floats2half2_rn(a, b);
-    return *reinterpret_cast<uint32_t*>(&h);
-  }
+  grouped_tile(u, p.num_units / p.n_tiles_n, p.n_tiles_n, p.gn, m_blk, n_blk);
 }
 
 // (a & b) | c in one LOP3
@@ -108,17 +95,14 @@ __device__ __forceinline__ uint32_t sub_mul2(uint32_t x2, uint32_t zm2, uint32_t
   }
 }
 
-template <bool kBf16, int kBits, int NG>
-__global__ void __launch_bounds__(Cfg<kBits, NG>::kThreads, 1)
+template <bool kBf16, int kBits>
+__global__ void __launch_bounds__(kThreads, 1)
 w4a16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmP,
                   const Params p) {
-  using C = Cfg<kBits, NG>;
+  using C = Cfg<kBits>;
   constexpr int kLStages = C::kLStages;
   constexpr int kLBytes = C::kLBytes;
-  constexpr int kBStages = C::kBStages;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
-                                             ~static_cast<uintptr_t>(1023));
+  uint8_t* smem = smem_align1024();
   uint8_t* ringL = smem;
   uint8_t* ringB = smem + kLStages * kLBytes;
   uint64_t* fullL = reinterpret_cast<uint64_t*>(ringB + kBStages * kBBytes);
@@ -144,65 +128,58 @@ w4a16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     for (int s = 0; s < 2; ++s) { mbar_init(&tmem_full[s], 1); mbar_init(&tmem_empty[s], 4); }
     fence_barrier_init();
   }
-  if (warp == 1) tmem_alloc(tmem_ptr, kTmemCols);
-  tcgen05_fence_before();
-  __syncthreads();
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
+  const uint32_t tmem_base = tmem_setup(warp, tmem_ptr, kTmemCols);
 
   if (warp == 0) {
     // ===================== TMA producer =====================
     if (lane == 0) {
-      int sl = 0;
-      uint32_t phl = 0;
+      Ring<kLStages> sl;
       for (int u = blockIdx.x; u < p.num_units; u += gridDim.x) {
         int m_blk, n_blk;
         decode(p, u, m_blk, n_blk);
         for (int kb = 0; kb < p.kb_total; ++kb) {
-          mbar_wait(&emptyL[sl], phl ^ 1);
-          uint8_t* a_dst = ringL + sl * kLBytes;
+          mbar_wait(&emptyL[sl.idx], sl.phase ^ 1);
+          uint8_t* a_dst = ringL + sl.idx * kLBytes;
           uint8_t* p_dst = a_dst + kABytes;
-          mbar_expect_tx(&fullL[sl], kLBytes);
-          tma_load_2d(a_dst, &tmA, &fullL[sl], kb * BK, m_blk * BM);
-          tma_load_2d(p_dst, &tmP, &fullL[sl], kb * C::kWordsPerRow, n_blk * BN);
-          if (++sl == kLStages) { sl = 0; phl ^= 1; }
+          mbar_expect_tx(&fullL[sl.idx], kLBytes);
+          tma_load_2d(a_dst, &tmA, &fullL[sl.idx], kb * BK, m_blk * BM);
+          tma_load_2d(p_dst, &tmP, &fullL[sl.idx], kb * C::kWordsPerRow, n_blk * BN);
+          sl.advance();
         }
       }
     }
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
-    constexpr uint32_t idesc = make_idesc_f16(kBf16 ? 1 : 0, 0, 0, BM, BN);
-    int sl = 0, sb = 0;
-    uint32_t phl = 0, phb = 0;
-    int as = 0;
-    uint32_t aphase = 0;
+    constexpr uint32_t idesc = make_idesc(kBf16, kBf16, 0, 0, BM, BN);
+    Ring<kLStages> sl;
+    Ring<kBStages> sb;
+    Ring<2> acc;
     for (int u = blockIdx.x; u < p.num_units; u += gridDim.x) {
-      mbar_wait(&tmem_empty[as], aphase ^ 1);
+      mbar_wait(&tmem_empty[acc.idx], acc.phase ^ 1);
       tcgen05_fence_after();
-      const uint32_t d_tmem = tmem_base + as * BN;
+      const uint32_t d_tmem = tmem_base + acc.idx * BN;
       for (int kb = 0; kb < p.kb_total; ++kb) {
-        mbar_wait(&fullL[sl], phl);              // X tile landed
-        mbar_wait(&readyB[sb], phb);             // W tile dequantised
+        mbar_wait(&fullL[sl.idx], sl.phase);     // X tile landed
+        mbar_wait(&readyB[sb.idx], sb.phase);    // W tile dequantised
         tcgen05_fence_after();
         if (lane == 0) {
-          const uint32_t a_addr = smem_u32(ringL + sl * kLBytes);
-          const uint32_t b_addr = smem_u32(ringB + sb * kBBytes);
+          const uint32_t a_addr = smem_u32(ringL + sl.idx * kLBytes);
+          const uint32_t b_addr = smem_u32(ringB + sb.idx * kBBytes);
 #pragma unroll
           for (int k = 0; k < BK / 16; ++k) {
             const uint64_t adesc = make_smem_desc(a_addr + k * 32, 16, 1024);
             const uint64_t bdesc = make_smem_desc(b_addr + k * 32, 16, 1024);
             umma_f16(d_tmem, adesc, bdesc, idesc, (kb > 0 || k > 0) ? 1u : 0u);
           }
-          umma_commit(&emptyL[sl]);
-          umma_commit(&emptyB[sb]);
-          if (kb == p.kb_total - 1) umma_commit(&tmem_full[as]);
+          umma_commit(&emptyL[sl.idx]);
+          umma_commit(&emptyB[sb.idx]);
+          if (kb == p.kb_total - 1) umma_commit(&tmem_full[acc.idx]);
         }
         __syncwarp();
-        if (++sl == kLStages) { sl = 0; phl ^= 1; }
-        if (++sb == kBStages) { sb = 0; phb ^= 1; }
+        sl.advance();
+        sb.advance();
       }
-      as ^= 1;
-      if (as == 0) aphase ^= 1;
+      acc.advance();
     }
   } else if (warp >= 6) {
     // ===================== dequant warps (4 * NG): two weight rows per thread =====================
@@ -210,7 +187,7 @@ w4a16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     // for its 128 weights of a tile is ~2300 cycles of dependent latency (round-2 finding: with two
     // groups the kernel ran at exactly one tile per two such chains, tensor pipe 44 % active, while
     // only half of the issue slots were used) — more groups in flight, not more instructions per
-    // clock, is what hides it.  Ring B has one stage per group.
+    // clock, is what hides it.
     const int grp = (warp - 6) % NG;
     const int tig = ((warp - 6) / NG) * 32 + lane;   // 0..127 inside the group
     uint32_t it = 0;                                 // K steps issued so far (all tiles)
@@ -356,73 +333,41 @@ w4a16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   } else {
     // ===================== epilogue (warps 2..5) =====================
     const int q = warp & 3;
-    int as = 0;
-    uint32_t aphase = 0;
+    Ring<2> acc;
     for (int u = blockIdx.x; u < p.num_units; u += gridDim.x) {
       int m_blk, n_blk;
       decode(p, u, m_blk, n_blk);
-      mbar_wait(&tmem_full[as], aphase);
+      mbar_wait(&tmem_full[acc.idx], acc.phase);
       tcgen05_fence_after();
       const int64_t row = static_cast<int64_t>(m_blk) * BM + q * 32 + lane;
-      const uint32_t taddr0 = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + as * BN;
+      const uint32_t taddr0 = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc.idx * BN;
 #pragma unroll 1
       for (int c = 0; c < BN; c += 32) {
         uint32_t r[32];
         tmem_ld_32x32b_x32(taddr0 + c, r);
         tmem_ld_wait();
         const int64_t col0 = static_cast<int64_t>(n_blk) * BN + c;
-        if (row < p.M && col0 < p.N) {
-          uint16_t* o = reinterpret_cast<uint16_t*>(p.out) + row * p.N + col0;
-          const uint16_t* bs = reinterpret_cast<const uint16_t*>(p.bias);
-          const bool full = (col0 + 32 <= p.N) && ((p.N & 7) == 0);
-          uint32_t pk[16];
-#pragma unroll
-          for (int i = 0; i < 32; i += 2) {
-            float v0 = __uint_as_float(r[i]), v1 = __uint_as_float(r[i + 1]);
-            if (bs != nullptr) {
-              if (col0 + i < p.N) v0 += kBf16 ? __uint_as_float(static_cast<uint32_t>(bs[col0 + i]) << 16)
-                                              : __half2float(__ushort_as_half(bs[col0 + i]));
-              if (col0 + i + 1 < p.N) v1 += kBf16 ? __uint_as_float(static_cast<uint32_t>(bs[col0 + i + 1]) << 16)
-                                                  : __half2float(__ushort_as_half(bs[col0 + i + 1]));
-            }
-            pk[i >> 1] = pack2<kBf16>(v0, v1);
-          }
-          if (full) {
-#pragma unroll
-            for (int i = 0; i < 16; i += 4)
-              *reinterpret_cast<uint4*>(o + 2 * i) = make_uint4(pk[i], pk[i + 1], pk[i + 2], pk[i + 3]);
-          } else {
-            for (int i = 0; i < 32 && col0 + i < p.N; ++i)
-              o[i] = static_cast<uint16_t>((i & 1) ? (pk[i >> 1] >> 16) : (pk[i >> 1] & 0xffffu));
-          }
-        }
+        if (row < p.M && col0 < p.N)
+          store_chunk_bias<kBf16>(reinterpret_cast<uint16_t*>(p.out) + row * p.N + col0, r,
+                                  reinterpret_cast<const uint16_t*>(p.bias), col0, p.N,
+                                  (p.N & 7) == 0);
       }
       tcgen05_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive(&tmem_empty[as]);
-      as ^= 1;
-      if (as == 0) aphase ^= 1;
+      if (lane == 0) mbar_arrive(&tmem_empty[acc.idx]);
+      acc.advance();
     }
   }
-  tcgen05_fence_before();
-  __syncthreads();
-  if (warp == 1) tmem_dealloc(tmem_base, kTmemCols);
+  tmem_teardown(warp, tmem_base, kTmemCols);
 }
 
 }  // namespace w4
-
-int encode_tmap_2d_b16(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
-                       uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols);
-int encode_tmap_2d_i32_noswizzle(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
-                                 uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols,
-                                 int swizzle32);
-
 }  // namespace llmc
 
 using namespace llmc;
 
-template <int kBits, int NG>
-static int gemm_wNa16_ng(const void* x, const int32_t* wq, const void* scales, const void* zeros,
+template <int kBits>
+static int gemm_wNa16(const void* x, const int32_t* wq, const void* scales, const void* zeros,
                       int qparam_dtype, const void* bias, void* y, int64_t M, int64_t N, int64_t K,
                       int64_t group, int dtype, int q_transposed, void* stream, const char* name) {
   using namespace w4;
@@ -439,13 +384,16 @@ static int gemm_wNa16_ng(const void* x, const int32_t* wq, const void* scales, c
     set_last_error("%s: K=%lld must be a multiple of 64 and pointers 16-byte aligned", name, (long long)K);
     return LLMC_EALIGN;
   }
-  using C = Cfg<kBits, NG>;
-  constexpr int wpr = C::kWordsPerRow;
-  constexpr int kThreads = C::kThreads;
+  using C = Cfg<kBits>;
   CUtensorMap tmA, tmP;
-  if (int rc = encode_tmap_2d_b16(&tmA, x, M, K, K, BM, BK)) return rc;
-  if (int rc = encode_tmap_2d_i32_noswizzle(&tmP, wq, N, K * kBits / 32, K * kBits / 32, BN, wpr,
-                                            kBits == 4 ? 1 : 2))
+  if (int rc = encode_tmap_2d(&tmA, x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, M, K, K, BM, BK,
+                              CU_TENSOR_MAP_SWIZZLE_128B))
+    return rc;
+  // packed rows of 32 B (INT4) / 64 B (INT8): the 32B / 64B swizzle makes the dequant warps'
+  // one-row-per-thread 16-byte shared-memory loads conflict free
+  if (int rc = encode_tmap_2d(&tmP, wq, CU_TENSOR_MAP_DATA_TYPE_INT32, 4, N, K * kBits / 32,
+                              K * kBits / 32, BN, C::kWordsPerRow,
+                              kBits == 4 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_64B))
     return rc;
   Params p{};
   p.M = M; p.N = N; p.K = K; p.out = y; p.bias = bias;
@@ -460,36 +408,15 @@ static int gemm_wNa16_ng(const void* x, const int32_t* wq, const void* scales, c
   LLMC_CHECK_ARG(mt * p.n_tiles_n < (1ll << 31), "%s: too many tiles", name);
   p.num_units = static_cast<int>(mt * p.n_tiles_n);
   p.kb_total = static_cast<int>(K / BK);
-  {
-    int64_t gn = (32ll << 20) / (static_cast<int64_t>(BN) * K * kBits / 8 + 1);
-    if (gn < 1) gn = 1;
-    if (gn > p.n_tiles_n) gn = p.n_tiles_n;
-    p.gn = static_cast<int>(gn);
-  }
+  p.gn = raster_group_n(static_cast<int64_t>(BN) * K * kBits / 8, p.n_tiles_n);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   constexpr int smem = C::kSmemBytes;
   static_assert(smem <= 227 * 1024, "shared memory budget");
-  LLMC_ONCE_PER_DEVICE({
-    LLMC_CHECK_CUDA(cudaFuncSetAttribute(w4a16_gemm_kernel<true, kBits, NG>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    LLMC_CHECK_CUDA(cudaFuncSetAttribute(w4a16_gemm_kernel<false, kBits, NG>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  });
   const int grid = p.num_units < kNumSMs ? p.num_units : kNumSMs;
-  if (dtype == LLMC_BF16) w4a16_gemm_kernel<true, kBits, NG><<<grid, kThreads, smem, st>>>(tmA, tmP, p);
-  else w4a16_gemm_kernel<false, kBits, NG><<<grid, kThreads, smem, st>>>(tmA, tmP, p);
-  LLMC_CHECK_LAUNCH();
-  return LLMC_OK;
+  return dtype == LLMC_BF16 ? launch_tc<w4a16_gemm_kernel<true, kBits>>(grid, kThreads, smem, st, tmA, tmP, p)
+                            : launch_tc<w4a16_gemm_kernel<false, kBits>>(grid, kThreads, smem, st, tmA, tmP, p);
 }
 
-// Two dequant groups.  (A four-group variant — the template parameter NG exists for it — was
-// tried in round 2 on the theory that the per-thread unpack chain, not issue bandwidth, limits the
-// kernel: it was slower, 728 vs 871 TFLOP/s, and is not instantiated.)
-template <int kBits>
-static int gemm_wNa16(const void* x, const int32_t* wq, const void* scales, const void* zeros,
-                      int qparam_dtype, const void* bias, void* y, int64_t M, int64_t N, int64_t K,
-                      int64_t group, int dtype, int q_transposed, void* stream, const char* name) {
-  return gemm_wNa16_ng<kBits, 2>(x, wq, scales, zeros, qparam_dtype, bias, y, M, N, K, group, dtype,
-                                 q_transposed, stream, name);
-}
 
 extern "C" int llmc_gemm_w4a16(const void* x, const int32_t* wq, const void* scales,
                                const void* zeros, int qparam_dtype, const void* bias, void* y,

@@ -13,6 +13,7 @@
 // order of the 128-deep trailing dot products differs from the CPU BLAS.
 #include "common.cuh"
 #include "spqr_row.cuh"
+#include "tf32.cuh"
 
 namespace llmc {
 
@@ -968,20 +969,6 @@ extern "C" int llmc_gptq_prepare(const float* H, int64_t C, const int64_t* perm,
   return LLMC_OK;
 }
 
-namespace llmc {
-int tf32x3_update(const float* Ahi, const float* Alo, int a_mn, int64_t lda, const float* Bhi,
-                  const float* Blo, int b_mn, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                  int64_t N, int K, int mode, int tri, int64_t row_off, int64_t col_off,
-                  float* Chi, float* Clo, cudaStream_t st);
-int tf32x3_update_grid(const float* Ahi, const float* Alo, int a_mn, int64_t lda, const float* Bhi,
-                       const float* Blo, int b_mn, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                       int64_t N, int K, int mode, int tri, int64_t row_off, int64_t col_off,
-                       float* Chi, float* Clo, int64_t split_rows, int64_t split_cols,
-                       int one_tile_per_cta, cudaStream_t st);
-int split_tf32(const float* x, int64_t rows, int64_t cols, int64_t ld, float* hi, float* lo,
-               int64_t ld_out, cudaStream_t st);
-}  // namespace llmc
-
 // The schedule shared by the GPTQ and SpQR sweeps: in-block kernel per 128 columns (launched by
 // `launch_inblock(i1, count, err, err_hi, err_lo, stream)`), lazy trailing updates per super-panel
 // and the look-ahead split of the bulk update.  `wide_dynamic_group`: the in-block kernel reads
@@ -1070,13 +1057,18 @@ static int sweep_schedule(float* W, const float* Hinv, int64_t R, int64_t C, int
       // B = Hinv rows (MN-major, ld C).  Inside the super-panel: this block's errors onto the
       // super-panel's remaining columns; at its end: all of its errors onto everything beyond.
       if (i2 < sp1) {
-        if (int rc = tf32x3_update(b_err_hi, b_err_lo, 1, Rpad, Hh + i1 * C + i2, Hl + i1 * C + i2,
-                                   1, C, W + i2, C, R, sp1 - i2, b_count, 0, 0, 0, 0, nullptr, nullptr, chain))
+        if (int rc = tf32x3_update({.Ahi = b_err_hi, .Alo = b_err_lo, .a_mn = 1, .lda = Rpad,
+                                    .Bhi = Hh + i1 * C + i2, .Blo = Hl + i1 * C + i2, .b_mn = 1, .ldb = C,
+                                    .C = W + i2, .ldc = C, .M = R, .N = sp1 - i2, .K = b_count,
+                                    .mode = 0},
+                                   chain))
           return rc;
       } else if (!lookahead) {
-        if (int rc = tf32x3_update(errh_base, errl_base, 1, Rpad, Hh + sp0 * C + sp1, Hl + sp0 * C + sp1,
-                                   1, C, W + sp1, C, R, C - sp1, static_cast<int>(sp1 - sp0), 0, 0, 0, 0,
-                                   nullptr, nullptr, chain))
+        if (int rc = tf32x3_update({.Ahi = errh_base, .Alo = errl_base, .a_mn = 1, .lda = Rpad,
+                                    .Bhi = Hh + sp0 * C + sp1, .Blo = Hl + sp0 * C + sp1, .b_mn = 1, .ldb = C,
+                                    .C = W + sp1, .ldc = C, .M = R, .N = C - sp1,
+                                    .K = static_cast<int>(sp1 - sp0), .mode = 0},
+                                   chain))
           return rc;
       } else {
         const int kk = static_cast<int>(sp1 - sp0);
@@ -1085,16 +1077,20 @@ static int sweep_schedule(float* W, const float* Hinv, int64_t R, int64_t C, int
         LLMC_CHECK_CUDA(cudaEventRecord(panel_of[dev_id][par], chain));
         // chain: the next super-panel's columns, last written by the previous panel's bulk piece
         if (bulk_pending[par ^ 1]) LLMC_CHECK_CUDA(cudaStreamWaitEvent(chain, bulkdone_of[dev_id][par ^ 1], 0));
-        if (int rc = tf32x3_update(errh_base, errl_base, 1, Rpad, Hh + sp0 * C + sp1, Hl + sp0 * C + sp1,
-                                   1, C, W + sp1, C, R, nx1 - sp1, kk, 0, 0, 0, 0, nullptr, nullptr, chain))
+        if (int rc = tf32x3_update({.Ahi = errh_base, .Alo = errl_base, .a_mn = 1, .lda = Rpad,
+                                    .Bhi = Hh + sp0 * C + sp1, .Blo = Hl + sp0 * C + sp1, .b_mn = 1, .ldb = C,
+                                    .C = W + sp1, .ldc = C, .M = R, .N = nx1 - sp1, .K = kk, .mode = 0},
+                                   chain))
           return rc;
         // bulk: everything beyond.  After this wait the chain goes on to write the OTHER error set,
         // which the previous bulk piece (just waited for) was the last reader of.
         if (nx1 < C) {
           LLMC_CHECK_CUDA(cudaStreamWaitEvent(bulk, panel_of[dev_id][par], 0));
-          if (int rc = tf32x3_update_grid(errh_base, errl_base, 1, Rpad, Hh + sp0 * C + nx1, Hl + sp0 * C + nx1,
-                                          1, C, W + nx1, C, R, C - nx1, kk, 0, 0, 0, 0, nullptr, nullptr,
-                                          0, 0, 1, bulk))
+          if (int rc = tf32x3_update({.Ahi = errh_base, .Alo = errl_base, .a_mn = 1, .lda = Rpad,
+                                      .Bhi = Hh + sp0 * C + nx1, .Blo = Hl + sp0 * C + nx1, .b_mn = 1, .ldb = C,
+                                      .C = W + nx1, .ldc = C, .M = R, .N = C - nx1, .K = kk, .mode = 0,
+                                      .one_tile_per_cta = 1},
+                                     bulk))
             return rc;
           LLMC_CHECK_CUDA(cudaEventRecord(bulkdone_of[dev_id][par], bulk));
           bulk_pending[par] = true;

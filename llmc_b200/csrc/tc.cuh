@@ -1,6 +1,9 @@
 // tc.cuh — sm_100a building blocks: mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (UMMA +
 // TMEM).  Hand-written inline PTX; bit layouts follow the PTX ISA "tcgen05" chapter
-// (cross-checked against cute/arch/mma_sm100_desc.hpp field tables).
+// (cross-checked against cute/arch/mma_sm100_desc.hpp field tables).  Also the scaffolding the
+// persistent warp-specialised kernels share (gemm.cu, tf32.cu, gemm_w4.cu, gemm_fp8.cu): smem
+// alignment, TMEM setup / teardown, ring positions, grouped rasterisation, the bf16 / fp16
+// epilogue stores, the tensor-map encoder and the launch helper.
 #pragma once
 
 #include <cuda.h>  // CUtensorMap (types only; the driver entry point is resolved at run time)
@@ -160,16 +163,19 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t lbo_
   return d;
 }
 
-// Instruction descriptor for kind::f16 (fp16/bf16 inputs, fp32 accumulate):
-//   [4,6) D format: 1 = f32      [7,10) A format: 0 = f16, 1 = bf16     [10,13) B format
-//   [15] A major: 0 = K, 1 = MN  [16] B major     [17,23) N >> 3        [24,29) M >> 4
-__host__ __device__ constexpr uint32_t make_idesc_f16(int bf16, int a_mn, int b_mn, int M, int N) {
-  return (1u << 4) | (static_cast<uint32_t>(bf16) << 7) | (static_cast<uint32_t>(bf16) << 10) |
+// Instruction descriptor (fp32 accumulate), the same field layout for every MMA kind:
+//   [4,6) D format: 1 = f32      [7,10) A format      [10,13) B format
+//   [15] A major: 0 = K, 1 = MN  [16] B major         [17,23) N >> 3        [24,29) M >> 4
+// Format codes per kind: kind::f16 0 = f16, 1 = bf16; kind::tf32 2 = tf32; kind::f8f6f4 0 = e4m3.
+__host__ __device__ constexpr uint32_t make_idesc(int a_fmt, int b_fmt, int a_mn, int b_mn, int M,
+                                                  int N) {
+  return (1u << 4) | (static_cast<uint32_t>(a_fmt) << 7) | (static_cast<uint32_t>(b_fmt) << 10) |
          (static_cast<uint32_t>(a_mn) << 15) | (static_cast<uint32_t>(b_mn) << 16) |
          (static_cast<uint32_t>(N >> 3) << 17) | (static_cast<uint32_t>(M >> 4) << 24);
 }
 
-// D[tmem] (+)= A[smem] * B[smem], issued by ONE thread.
+// D[tmem] (+)= A[smem] * B[smem], issued by ONE thread.  K per instruction: 16 (f16 / bf16),
+// 8 (tf32), 32 (8-bit operands).
 __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc,
                                          uint32_t idesc, uint32_t accumulate) {
   asm volatile(
@@ -181,14 +187,17 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-
-// Instruction descriptor for kind::f8f6f4 with E4M3 x E4M3 -> F32, both operands K-major.
-// Same field layout as kind::f16; the A/B format code 0 means E4M3 under this kind.
-__host__ __device__ constexpr uint32_t make_idesc_e4m3(int M, int N) {
-  return (1u << 4) | (static_cast<uint32_t>(N >> 3) << 17) | (static_cast<uint32_t>(M >> 4) << 24);
+__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc,
+                                          uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
 }
-
-// D[tmem] (+)= A[smem] * B[smem] for 8-bit operands (K = 32 per instruction), ONE thread.
 __device__ __forceinline__ void umma_f8f6f4(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc,
                                             uint32_t idesc, uint32_t accumulate) {
   asm volatile(
@@ -199,6 +208,106 @@ __device__ __forceinline__ void umma_f8f6f4(uint32_t tmem_d, uint64_t adesc, uin
       "}\n" ::"r"(tmem_d),
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
+}
+
+// ---- persistent-kernel scaffolding -------------------------------------------------------------
+// Dynamic shared memory, rounded up to the 1024-byte alignment of 128B-swizzle atoms (kernels
+// reserve 1024 bytes of slack for it).
+__device__ __forceinline__ uint8_t* smem_align1024() {
+  extern __shared__ uint8_t smem_raw[];
+  return reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
+                                    ~static_cast<uintptr_t>(1023));
+}
+
+// Called by every thread after the barriers are initialised: warp 1 allocates `ncols` TMEM
+// columns, the barrier initialisation and the allocation become visible to all threads, and the
+// TMEM base address is returned.  `warp` = threadIdx.x / 32.
+__device__ __forceinline__ uint32_t tmem_setup(int warp, uint32_t* tmem_ptr, uint32_t ncols) {
+  if (warp == 1) tmem_alloc(tmem_ptr, ncols);
+  tcgen05_fence_before();
+  __syncthreads();
+  tcgen05_fence_after();
+  return *tmem_ptr;
+}
+// Called by every thread at the end: warp 1 frees the columns once all TMEM traffic is done.
+__device__ __forceinline__ void tmem_teardown(int warp, uint32_t tmem_base, uint32_t ncols) {
+  tcgen05_fence_before();
+  __syncthreads();
+  if (warp == 1) tmem_dealloc(tmem_base, ncols);
+}
+
+// Position in a ring of kN mbarrier-guarded slots: slot index and the parity of the current pass.
+template <int kN>
+struct Ring {
+  int idx = 0;
+  uint32_t phase = 0;
+  __device__ __forceinline__ void advance() {
+    if (++idx == kN) { idx = 0; phase ^= 1; }
+  }
+};
+
+// Grouped rasterisation of an m_tiles x n_tiles output: the weights (n) are swept in groups of
+// `gn` n-tiles sized to stay L2-resident (raster_group_n), all m-tiles per group, n fastest
+// inside the group.  Activations are re-read once per group from HBM, weights once; n-fastest
+// over the whole N would instead stream every weight through L2 once per wave of tiles.
+__device__ __forceinline__ void grouped_tile(int u, int m_tiles, int n_tiles, int gn, int& m_blk,
+                                             int& n_blk) {
+  const int per_group = gn * m_tiles;
+  const int g = u / per_group;
+  const int rem = u - g * per_group;
+  const int gsz = min(gn, n_tiles - g * gn);
+  m_blk = rem / gsz;
+  n_blk = g * gn + (rem - m_blk * gsz);
+}
+
+// ---- bf16 / fp16 epilogue ---------------------------------------------------------------------
+template <bool kBf16>
+__device__ __forceinline__ uint32_t pack2(float a, float b) {
+  if constexpr (kBf16) {
+    __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+    return *reinterpret_cast<uint32_t*>(&h);
+  } else {
+    __half2 h = __floats2half2_rn(a, b);
+    return *reinterpret_cast<uint32_t*>(&h);
+  }
+}
+
+// Columns [col0, col0 + 32) of a row of 16-bit outputs (`o` points at column col0), packed in
+// pairs: four 16-byte stores when `full` (all 32 columns inside the row and the row 16-byte
+// aligned), else the columns below N one by one.
+__device__ __forceinline__ void store_row32_b16(uint16_t* o, const uint32_t (&pk)[16], bool full,
+                                                int64_t col0, int64_t N) {
+  if (full) {
+#pragma unroll
+    for (int i = 0; i < 16; i += 4)
+      *reinterpret_cast<uint4*>(o + 2 * i) = make_uint4(pk[i], pk[i + 1], pk[i + 2], pk[i + 3]);
+  } else {
+#pragma unroll
+    for (int i = 0; i < 32 && col0 + i < N; ++i)
+      o[i] = static_cast<uint16_t>((i & 1) ? (pk[i >> 1] >> 16) : (pk[i >> 1] & 0xffffu));
+  }
+}
+
+// One 32-column chunk of fp32 accumulators -> T (bf16 / fp16): columns [col0, col0 + 32) of a row
+// at `o`, masked to col < N.  bias[col] (T, may be null) is added in fp32 before the single
+// rounding, as F.linear does.  `ld_aligned`: rows start 16-byte aligned.
+template <bool kBf16>
+__device__ __forceinline__ void store_chunk_bias(uint16_t* o, const uint32_t (&r)[32],
+                                                 const uint16_t* bias, int64_t col0, int64_t N,
+                                                 bool ld_aligned) {
+  uint32_t pk[16];
+#pragma unroll
+  for (int i = 0; i < 32; i += 2) {
+    float v0 = __uint_as_float(r[i]), v1 = __uint_as_float(r[i + 1]);
+    if (bias != nullptr) {
+      if (col0 + i < N) v0 += kBf16 ? __uint_as_float(static_cast<uint32_t>(bias[col0 + i]) << 16)
+                                    : __half2float(__ushort_as_half(bias[col0 + i]));
+      if (col0 + i + 1 < N) v1 += kBf16 ? __uint_as_float(static_cast<uint32_t>(bias[col0 + i + 1]) << 16)
+                                        : __half2float(__ushort_as_half(bias[col0 + i + 1]));
+    }
+    pk[i >> 1] = pack2<kBf16>(v0, v1);
+  }
+  store_row32_b16(o, pk, col0 + 32 <= N && ld_aligned, col0, N);
 }
 
 // Packed fp32 pair arithmetic (sm_100): (c0, c1) = fma((d0, d1) * sa, sb, (c0, c1)), with the
@@ -221,13 +330,34 @@ __device__ __forceinline__ void promote2(float& c0, float& c1, float d0, float d
 
 }  // namespace tc
 
-// ---- host: tensor-map encoding through the driver entry point ---------------------------------
-// rows x cols matrix of 2-byte elements, row stride ld_elems; box = box_cols (inner) x box_rows,
-// 128-byte swizzle (box_cols * 2 must be 128).
-int encode_tmap_2d_b16(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
-                       uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols);
-// The same for 1-byte elements (fp8): box_cols must be 128.
-int encode_tmap_2d_u8(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
-                      uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols);
+// ---- host ------------------------------------------------------------------------------------
+// Tensor map of a row-major rows x cols matrix of `elem_bytes`-byte elements with row stride
+// ld_elems; box = box_cols (inner) x box_rows.  The swizzle span bounds the box's inner extent:
+// box_cols * elem_bytes must be 128 for SWIZZLE_128B(_ATOM_32B), 64 for 64B, 32 for 32B.
+// Encoded through the driver entry point resolved at run time (the library links no libcuda).
+int encode_tmap_2d(CUtensorMap* out, const void* base, CUtensorMapDataType dtype,
+                   uint32_t elem_bytes, uint64_t rows, uint64_t cols, uint64_t ld_elems,
+                   uint32_t box_rows, uint32_t box_cols, CUtensorMapSwizzle swizzle);
+
+// Weight-group width of grouped_tile: as many n-tiles as fit in ~32 MiB (L2-resident), at least
+// one and at most all of them.
+inline int raster_group_n(int64_t n_tile_bytes, int n_tiles_n) {
+  int64_t gn = (32ll << 20) / n_tile_bytes;
+  if (gn < 1) gn = 1;
+  if (gn > n_tiles_n) gn = n_tiles_n;
+  return static_cast<int>(gn);
+}
+
+// Launch a tcgen05 kernel on `grid` CTAs: the first launch on each device opts in to `smem` bytes
+// of dynamic shared memory (one flag per kernel instantiation), and every launch is counted.
+template <auto kKernel, typename... Args>
+int launch_tc(int grid, int threads, int smem, cudaStream_t st, const Args&... args) {
+  LLMC_ONCE_PER_DEVICE({
+    LLMC_CHECK_CUDA(cudaFuncSetAttribute(kKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  });
+  kKernel<<<grid, threads, smem, st>>>(args...);
+  LLMC_CHECK_LAUNCH();
+  return LLMC_OK;
+}
 
 }  // namespace llmc

@@ -16,8 +16,10 @@
 //   K-major : element (i, k) at base[i*ld + k]   (rows = M or N index, K contiguous)
 //   MN-major: element (i, k) at base[k*ld + i]   (rows = K index, M or N contiguous)
 // Same warp-specialised structure as gemm.cu (TMA producer / MMA issuer / 4 epilogue warps,
-// double-buffered 2 x 256-column TMEM accumulators), tile 128 x 256, 32 k per stage, 2 stages.
+// double-buffered 2 x 256-column TMEM accumulators, scaffolding from tc.cuh), tile 128 x 256,
+// 32 k per stage, 2 stages.  Host entry point: tf32x3_update(const Tf32x3Update&) in tf32.cuh.
 #include "tc.cuh"
+#include "tf32.cuh"
 
 namespace llmc {
 
@@ -71,25 +73,6 @@ __device__ __forceinline__ void decode(const Params& p, int u, int& m_blk, int& 
   n_blk = u;
 }
 
-// Instruction descriptor kind::tf32: D f32 (1<<4), A/B format 2 = TF32.
-__host__ __device__ constexpr uint32_t idesc_tf32(int a_mn, int b_mn) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | (static_cast<uint32_t>(a_mn) << 15) |
-         (static_cast<uint32_t>(b_mn) << 16) | (static_cast<uint32_t>(BN >> 3) << 17) |
-         (static_cast<uint32_t>(BM >> 4) << 24);
-}
-
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc,
-                                          uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
-      "}\n" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
 __device__ __forceinline__ float to_tf32(float x) {
   uint32_t r;
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
@@ -101,9 +84,7 @@ __global__ void __launch_bounds__(kThreads, 1)
 tf32x3_kernel(const __grid_constant__ CUtensorMap tmAhi, const __grid_constant__ CUtensorMap tmAlo,
               const __grid_constant__ CUtensorMap tmBhi, const __grid_constant__ CUtensorMap tmBlo,
               const Params p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
-                                             ~static_cast<uintptr_t>(1023));
+  uint8_t* smem = smem_align1024();
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + kStages * kStageBytes);
   uint64_t* empty_bar = full_bar + kStages;
   uint64_t* tmem_full = empty_bar + kStages;
@@ -118,65 +99,59 @@ tf32x3_kernel(const __grid_constant__ CUtensorMap tmAhi, const __grid_constant__
     for (int s = 0; s < 2; ++s) { mbar_init(&tmem_full[s], 1); mbar_init(&tmem_empty[s], 4); }
     fence_barrier_init();
   }
-  if (warp == 1) tmem_alloc(tmem_ptr, kTmemCols);
-  tcgen05_fence_before();
-  __syncthreads();
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
+  const uint32_t tmem_base = tmem_setup(warp, tmem_ptr, kTmemCols);
 
   if (warp == 0) {
     if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
+      Ring<kStages> s;
       for (int u = blockIdx.x; u < p.num_units; u += gridDim.x) {
         int m_blk, n_blk;
         decode(p, u, m_blk, n_blk);
         for (int kb = 0; kb < kb_total; ++kb) {
-          mbar_wait(&empty_bar[stage], phase ^ 1);
-          uint8_t* ahi = smem + stage * kStageBytes;
+          mbar_wait(&empty_bar[s.idx], s.phase ^ 1);
+          uint8_t* ahi = smem + s.idx * kStageBytes;
           uint8_t* alo = ahi + kABytes;
           uint8_t* bhi = alo + kABytes;
           uint8_t* blo = bhi + kBBytes;
-          mbar_expect_tx(&full_bar[stage], kStageBytes);
+          uint64_t* bar = &full_bar[s.idx];
+          mbar_expect_tx(bar, kStageBytes);
           if constexpr (!kAmn) {
-            tma_load_2d(ahi, &tmAhi, &full_bar[stage], kb * BK, m_blk * BM);
-            tma_load_2d(alo, &tmAlo, &full_bar[stage], kb * BK, m_blk * BM);
+            tma_load_2d(ahi, &tmAhi, bar, kb * BK, m_blk * BM);
+            tma_load_2d(alo, &tmAlo, bar, kb * BK, m_blk * BM);
           } else {
 #pragma unroll
             for (int i = 0; i < BM / 32; ++i) {
-              tma_load_2d(ahi + i * kBoxBytes, &tmAhi, &full_bar[stage], m_blk * BM + i * 32, kb * BK);
-              tma_load_2d(alo + i * kBoxBytes, &tmAlo, &full_bar[stage], m_blk * BM + i * 32, kb * BK);
+              tma_load_2d(ahi + i * kBoxBytes, &tmAhi, bar, m_blk * BM + i * 32, kb * BK);
+              tma_load_2d(alo + i * kBoxBytes, &tmAlo, bar, m_blk * BM + i * 32, kb * BK);
             }
           }
           if constexpr (!kBmn) {
-            tma_load_2d(bhi, &tmBhi, &full_bar[stage], kb * BK, n_blk * BN);
-            tma_load_2d(blo, &tmBlo, &full_bar[stage], kb * BK, n_blk * BN);
+            tma_load_2d(bhi, &tmBhi, bar, kb * BK, n_blk * BN);
+            tma_load_2d(blo, &tmBlo, bar, kb * BK, n_blk * BN);
           } else {
 #pragma unroll
             for (int i = 0; i < BN / 32; ++i) {
-              tma_load_2d(bhi + i * kBoxBytes, &tmBhi, &full_bar[stage], n_blk * BN + i * 32, kb * BK);
-              tma_load_2d(blo + i * kBoxBytes, &tmBlo, &full_bar[stage], n_blk * BN + i * 32, kb * BK);
+              tma_load_2d(bhi + i * kBoxBytes, &tmBhi, bar, n_blk * BN + i * 32, kb * BK);
+              tma_load_2d(blo + i * kBoxBytes, &tmBlo, bar, n_blk * BN + i * 32, kb * BK);
             }
           }
-          if (++stage == kStages) { stage = 0; phase ^= 1; }
+          s.advance();
         }
       }
     }
   } else if (warp == 1) {
-    constexpr uint32_t idesc = idesc_tf32(kAmn ? 1 : 0, kBmn ? 1 : 0);
-    int stage = 0;
-    uint32_t phase = 0;
-    int as = 0;
-    uint32_t aphase = 0;
+    constexpr uint32_t idesc = make_idesc(2, 2, kAmn, kBmn, BM, BN);    // tf32 x tf32
+    Ring<kStages> s;
+    Ring<2> acc;
     for (int u = blockIdx.x; u < p.num_units; u += gridDim.x) {
-      mbar_wait(&tmem_empty[as], aphase ^ 1);
+      mbar_wait(&tmem_empty[acc.idx], acc.phase ^ 1);
       tcgen05_fence_after();
-      const uint32_t d_tmem = tmem_base + as * BN;
+      const uint32_t d_tmem = tmem_base + acc.idx * BN;
       for (int kb = 0; kb < kb_total; ++kb) {
-        mbar_wait(&full_bar[stage], phase);
+        mbar_wait(&full_bar[s.idx], s.phase);
         tcgen05_fence_after();
         if (lane == 0) {
-          const uint32_t ahi = smem_u32(smem + stage * kStageBytes);
+          const uint32_t ahi = smem_u32(smem + s.idx * kStageBytes);
           const uint32_t alo = ahi + kABytes;
           const uint32_t bhi = alo + kABytes;
           const uint32_t blo = bhi + kBBytes;
@@ -197,26 +172,24 @@ tf32x3_kernel(const __grid_constant__ CUtensorMap tmAhi, const __grid_constant__
             umma_tf32(d_tmem, dal, dbh, idesc, 1u);
             umma_tf32(d_tmem, dah, dbl, idesc, 1u);
           }
-          umma_commit(&empty_bar[stage]);
-          if (kb == kb_total - 1) umma_commit(&tmem_full[as]);
+          umma_commit(&empty_bar[s.idx]);
+          if (kb == kb_total - 1) umma_commit(&tmem_full[acc.idx]);
         }
         __syncwarp();
-        if (++stage == kStages) { stage = 0; phase ^= 1; }
+        s.advance();
       }
-      as ^= 1;
-      if (as == 0) aphase ^= 1;
+      acc.advance();
     }
   } else {
     const int q = warp & 3;
-    int as = 0;
-    uint32_t aphase = 0;
+    Ring<2> acc;
     for (int u = blockIdx.x; u < p.num_units; u += gridDim.x) {
       int m_blk, n_blk;
       decode(p, u, m_blk, n_blk);
-      mbar_wait(&tmem_full[as], aphase);
+      mbar_wait(&tmem_full[acc.idx], acc.phase);
       tcgen05_fence_after();
       const int64_t row = static_cast<int64_t>(m_blk) * BM + q * 32 + lane;
-      const uint32_t taddr0 = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + as * BN;
+      const uint32_t taddr0 = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc.idx * BN;
 #pragma unroll 1
       for (int c = 0; c < BN; c += 32) {
         uint32_t r[32];
@@ -275,14 +248,11 @@ tf32x3_kernel(const __grid_constant__ CUtensorMap tmAhi, const __grid_constant__
       }
       tcgen05_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive(&tmem_empty[as]);
-      as ^= 1;
-      if (as == 0) aphase ^= 1;
+      if (lane == 0) mbar_arrive(&tmem_empty[acc.idx]);
+      acc.advance();
     }
   }
-  tcgen05_fence_before();
-  __syncthreads();
-  if (warp == 1) tmem_dealloc(tmem_base, kTmemCols);
+  tmem_teardown(warp, tmem_base, kTmemCols);
 }
 
 __global__ void __launch_bounds__(256)
@@ -301,106 +271,54 @@ split_tf32_kernel(const float* __restrict__ x, int64_t rows, int64_t cols, int64
 
 }  // namespace t3
 
-// rows x cols fp32 matrix, row stride ld; 128-byte swizzle => box_cols must be 32.
-int encode_tmap_2d_f32(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
-                       uint64_t ld_elems, uint32_t box_rows, uint32_t box_cols, int atom32b);
-
-// One 3xTF32 update.  a_mn / b_mn: operand is MN-major (element (i,k) at base[k*ld + i]).
-// split_rows / split_cols restrict where the tf32 split of the result (Chi/Clo) is written: rows
-// [0, split_rows) and columns [0, split_cols) of C (multiples of 32).  The blocked Cholesky uses
-// this to get the split of the *next* panel for free from the trailing update.
-int tf32x3_update_ex(const float* Ahi, const float* Alo, int a_mn, int64_t lda, const float* Bhi,
-                     const float* Blo, int b_mn, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                     int64_t N, int K, int mode, int tri, int64_t row_off, int64_t col_off,
-                     float* Chi, float* Clo, int64_t split_rows, int64_t split_cols,
-                     cudaStream_t st);
-int tf32x3_update_grid(const float* Ahi, const float* Alo, int a_mn, int64_t lda, const float* Bhi,
-                       const float* Blo, int b_mn, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                       int64_t N, int K, int mode, int tri, int64_t row_off, int64_t col_off,
-                       float* Chi, float* Clo, int64_t split_rows, int64_t split_cols,
-                       int one_tile_per_cta, cudaStream_t st);
-
-int tf32x3_update(const float* Ahi, const float* Alo, int a_mn, int64_t lda, const float* Bhi,
-                  const float* Blo, int b_mn, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                  int64_t N, int K, int mode, int tri, int64_t row_off, int64_t col_off,
-                  float* Chi, float* Clo, cudaStream_t st) {
-  return tf32x3_update_ex(Ahi, Alo, a_mn, lda, Bhi, Blo, b_mn, ldb, C, ldc, M, N, K, mode, tri,
-                          row_off, col_off, Chi, Clo, INT64_MAX, INT64_MAX, st);
-}
-
-int tf32x3_update_ex(const float* Ahi, const float* Alo, int a_mn, int64_t lda, const float* Bhi,
-                     const float* Blo, int b_mn, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                     int64_t N, int K, int mode, int tri, int64_t row_off, int64_t col_off,
-                     float* Chi, float* Clo, int64_t split_rows, int64_t split_cols,
-                     cudaStream_t st) {
-  return tf32x3_update_grid(Ahi, Alo, a_mn, lda, Bhi, Blo, b_mn, ldb, C, ldc, M, N, K, mode, tri,
-                            row_off, col_off, Chi, Clo, split_rows, split_cols, 0, st);
-}
-
-// one_tile_per_cta != 0: grid = number of tiles, every CTA computes one tile and exits.  Bulk
-// updates launched on a LOW-priority stream this way give their SMs back at tile granularity
-// (~20 us), so the short kernels of a latency-bound chain on a high-priority stream (blocked
-// Cholesky look-ahead, chol.cu) never wait behind a persistent 148-CTA grid.
-int tf32x3_update_grid(const float* Ahi, const float* Alo, int a_mn, int64_t lda, const float* Bhi,
-                       const float* Blo, int b_mn, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                       int64_t N, int K, int mode, int tri, int64_t row_off, int64_t col_off,
-                       float* Chi, float* Clo, int64_t split_rows, int64_t split_cols,
-                       int one_tile_per_cta, cudaStream_t st) {
+int tf32x3_update(const Tf32x3Update& u, cudaStream_t st) {
   using namespace t3;
+  const int64_t M = u.M, N = u.N;
+  const int K = u.K;
   if (M <= 0 || N <= 0 || K <= 0) return LLMC_OK;
-  if ((lda % 4) || (ldb % 4) || !aligned16(Ahi) || !aligned16(Alo) || !aligned16(Bhi) ||
-      !aligned16(Blo)) {
+  if ((u.lda % 4) || (u.ldb % 4) || !aligned16(u.Ahi) || !aligned16(u.Alo) || !aligned16(u.Bhi) ||
+      !aligned16(u.Blo)) {
     set_last_error("tf32x3_update: operands need 16-byte aligned bases and ld %% 4 == 0");
     return LLMC_EALIGN;
   }
+  // K-major: [rows, K] boxes of BK fp32 = 128 B, 128B swizzle; MN-major: [K, rows] boxes of
+  // 32 fp32, 128B swizzle with 32-byte atoms (SWIZZLE_128B_BASE32B in the smem descriptor)
+  auto encode = [&](CUtensorMap* m, const float* base, int mn, int64_t rows, int64_t ld,
+                    uint32_t box_rows) {
+    return mn ? encode_tmap_2d(m, base, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, K, rows, ld, BK, 32,
+                               CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B)
+              : encode_tmap_2d(m, base, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, rows, K, ld, box_rows,
+                               BK, CU_TENSOR_MAP_SWIZZLE_128B);
+  };
   CUtensorMap tah, tal, tbh, tbl;
-  int rc;
-  if (!a_mn) {
-    if ((rc = encode_tmap_2d_f32(&tah, Ahi, M, K, lda, BM, BK, 0))) return rc;
-    if ((rc = encode_tmap_2d_f32(&tal, Alo, M, K, lda, BM, BK, 0))) return rc;
-  } else {
-    if ((rc = encode_tmap_2d_f32(&tah, Ahi, K, M, lda, BK, 32, 1))) return rc;
-    if ((rc = encode_tmap_2d_f32(&tal, Alo, K, M, lda, BK, 32, 1))) return rc;
-  }
-  if (!b_mn) {
-    if ((rc = encode_tmap_2d_f32(&tbh, Bhi, N, K, ldb, BN, BK, 0))) return rc;
-    if ((rc = encode_tmap_2d_f32(&tbl, Blo, N, K, ldb, BN, BK, 0))) return rc;
-  } else {
-    if ((rc = encode_tmap_2d_f32(&tbh, Bhi, K, N, ldb, BK, 32, 1))) return rc;
-    if ((rc = encode_tmap_2d_f32(&tbl, Blo, K, N, ldb, BK, 32, 1))) return rc;
-  }
+  if (int rc = encode(&tah, u.Ahi, u.a_mn, M, u.lda, BM)) return rc;
+  if (int rc = encode(&tal, u.Alo, u.a_mn, M, u.lda, BM)) return rc;
+  if (int rc = encode(&tbh, u.Bhi, u.b_mn, N, u.ldb, BN)) return rc;
+  if (int rc = encode(&tbl, u.Blo, u.b_mn, N, u.ldb, BN)) return rc;
   Params p{};
-  p.M = M; p.N = N; p.K = K; p.C = C; p.ldc = ldc; p.Chi = Chi; p.Clo = Clo;
-  p.mode = mode; p.tri = tri; p.row_off = row_off; p.col_off = col_off;
-  p.split_rows = split_rows; p.split_cols = split_cols;
+  p.M = M; p.N = N; p.K = K; p.C = u.C; p.ldc = u.ldc; p.Chi = u.Chi; p.Clo = u.Clo;
+  p.mode = u.mode; p.tri = u.tri; p.row_off = u.row_off; p.col_off = u.col_off;
+  p.split_rows = u.split_rows; p.split_cols = u.split_cols;
   p.n_tiles_m = static_cast<int>((M + BM - 1) / BM);
   p.n_tiles_n = static_cast<int>((N + BN - 1) / BN);
-  if (!tri) {
+  if (!u.tri) {
     p.num_units = p.n_tiles_m * p.n_tiles_n;
   } else {
     long units = 0;
     for (int mi = 0; mi < p.n_tiles_m; ++mi) {
-      const int64_t last_row = row_off + static_cast<int64_t>(mi) * BM + BM - 1;
-      int64_t cnt = last_row < col_off ? 0 : (last_row - col_off) / BN + 1;
+      const int64_t last_row = u.row_off + static_cast<int64_t>(mi) * BM + BM - 1;
+      int64_t cnt = last_row < u.col_off ? 0 : (last_row - u.col_off) / BN + 1;
       if (cnt > p.n_tiles_n) cnt = p.n_tiles_n;
       units += cnt;
     }
     p.num_units = static_cast<int>(units);
   }
   if (p.num_units == 0) return LLMC_OK;
-  const int grid = (one_tile_per_cta || p.num_units < kNumSMs) ? p.num_units : kNumSMs;
-  LLMC_ONCE_PER_DEVICE({
-    LLMC_CHECK_CUDA(cudaFuncSetAttribute(tf32x3_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-    LLMC_CHECK_CUDA(cudaFuncSetAttribute(tf32x3_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-    LLMC_CHECK_CUDA(cudaFuncSetAttribute(tf32x3_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-    LLMC_CHECK_CUDA(cudaFuncSetAttribute(tf32x3_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  });
-  if (!a_mn && !b_mn) tf32x3_kernel<false, false><<<grid, kThreads, kSmemBytes, st>>>(tah, tal, tbh, tbl, p);
-  else if (!a_mn && b_mn) tf32x3_kernel<false, true><<<grid, kThreads, kSmemBytes, st>>>(tah, tal, tbh, tbl, p);
-  else if (a_mn && !b_mn) tf32x3_kernel<true, false><<<grid, kThreads, kSmemBytes, st>>>(tah, tal, tbh, tbl, p);
-  else tf32x3_kernel<true, true><<<grid, kThreads, kSmemBytes, st>>>(tah, tal, tbh, tbl, p);
-  LLMC_CHECK_LAUNCH();
-  return LLMC_OK;
+  const int grid = (u.one_tile_per_cta || p.num_units < kNumSMs) ? p.num_units : kNumSMs;
+  if (!u.a_mn && !u.b_mn) return launch_tc<tf32x3_kernel<false, false>>(grid, kThreads, kSmemBytes, st, tah, tal, tbh, tbl, p);
+  if (!u.a_mn && u.b_mn) return launch_tc<tf32x3_kernel<false, true>>(grid, kThreads, kSmemBytes, st, tah, tal, tbh, tbl, p);
+  if (u.a_mn && !u.b_mn) return launch_tc<tf32x3_kernel<true, false>>(grid, kThreads, kSmemBytes, st, tah, tal, tbh, tbl, p);
+  return launch_tc<tf32x3_kernel<true, true>>(grid, kThreads, kSmemBytes, st, tah, tal, tbh, tbl, p);
 }
 
 int split_tf32(const float* x, int64_t rows, int64_t cols, int64_t ld, float* hi, float* lo,
@@ -431,6 +349,9 @@ extern "C" int llmc_gemm_f32x3(const float* a_hi, const float* a_lo, int a_mn, i
   LLMC_CHECK_ARG(a_hi && a_lo && b_hi && b_lo && c, "gemm_f32x3: null pointer");
   LLMC_CHECK_ARG(M >= 0 && N >= 0 && K > 0 && K % 8 == 0 && K <= (1 << 20), "gemm_f32x3: bad shape (K %% 8 == 0)");
   LLMC_CHECK_ARG(mode == 0 || mode == 1, "gemm_f32x3: mode must be 0 (C -= AB) or 1 (C = AB)");
-  return tf32x3_update(a_hi, a_lo, a_mn, lda, b_hi, b_lo, b_mn, ldb, c, ldc, M, N, (int)K, mode,
-                       lower_only, 0, 0, nullptr, nullptr, static_cast<cudaStream_t>(stream));
+  return tf32x3_update({.Ahi = a_hi, .Alo = a_lo, .a_mn = a_mn, .lda = lda,
+                        .Bhi = b_hi, .Blo = b_lo, .b_mn = b_mn, .ldb = ldb,
+                        .C = c, .ldc = ldc, .M = M, .N = N, .K = (int)K, .mode = mode,
+                        .tri = lower_only},
+                       static_cast<cudaStream_t>(stream));
 }
